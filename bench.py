@@ -2,7 +2,7 @@
 """Benchmark of the ciMRGP VI hot path (BASELINE.json: VI iterations/sec at N = 1e6, 10 resolutions; batched
 Cholesky GFLOP/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" is one full variational sweep (`_fit()`, MRGP.py:571-652) over all 10 layers of the config-4 workload
 (N = 1e6 samples, dx = 1, dy = 2, M = 30, 1023 regions, ci mode, fp64, static basis intervals).  Prints ONE JSON line.
@@ -56,6 +56,32 @@ WORKLOAD = 'config4: synthetic 1-D nonstationary signal (script-1 f, seed 10), N
 CONFIG = {'workload': WORKLOAD, 'l2': 'GPU arm: L2 flushed between timed steps (256 MB write); CPU arm: n/a'}
 # algorithmic HBM bytes per sample-layer (SURVEY.md §8d): phase A 8(dx+2dy) = 40, phase B 8(dx+2dy+1) + 8(dy+1) = 72
 BYTES_SWEEP_PER_SAMPLE_LAYER = 112
+# --dump-outputs: the latent functions have one row per sample (240 MB at N = 1e6 over 10 layers); a fixed sample of
+# DUMP_ROWS rows keeps the whole dump near 35 MB, under DUMP_BYTES
+DUMP_ROWS = 1 << 17
+DUMP_BYTES = 64 << 20
+
+
+def engine_outputs(eng):
+    """What a caller reads back after a sweep: every array of Engine.state() (per-layer posteriors, shared Bingham / ARD /
+    omega state, latent functions) and the six ELBO terms per layer.  Per-sample arrays are cut to a seeded sample of rows,
+    whose indices are returned as `latent_rows`."""
+    rows = np.sort(np.random.RandomState(0).choice(eng.N, min(eng.N, DUMP_ROWS), replace=False))
+    out = {k: v[rows] if k.endswith(('.fbar', '.fvar')) else v for k, v in eng.state(latent=True).items()}
+    out['latent_rows'] = rows
+    out['elbo'] = eng.elbo()
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    """One float64 DIR/<name>.npy per array, so that two builds can be compared output for output."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_BYTES:
+        raise ValueError('outputs of %d bytes exceed the dump limit of %d' % (total, DUMP_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), v)
 
 
 def peaks():
@@ -139,9 +165,10 @@ def make_model(n, layers, device, fi=False, distributed=False, n_basis=N_BASIS, 
 # ------------------------------------------------------------------------------------------------------------------
 # CPU arms
 # ------------------------------------------------------------------------------------------------------------------
-def port_sweeps(n, layers, warmup, steps):
+def port_sweeps(n, layers, warmup, steps, dump=None):
     """The C restatement of the ci sweep (oracle/mrgp_port.c, OpenMP over all host threads) at FULL size n: seconds of
-    each of `steps` sweeps after `warmup` sweeps, the threads it used, the seconds of its constructor."""
+    each of `steps` sweeps after `warmup` sweeps, the threads it used, the seconds of its constructor.  dump: directory
+    that receives the state after the last sweep."""
     import workloads
     from oracle import mrgp_oracle as O
     from oracle import port_c
@@ -156,6 +183,8 @@ def port_sweeps(n, layers, warmup, steps):
         p.sweep(1)
         times.append(time.perf_counter() - t0)
     threads = p.threads
+    if dump:
+        dump_outputs(dump, p.state())
     p.close()
     return times, threads, t_ctor
 
@@ -228,7 +257,7 @@ def run_reference(args, rank, world):
     """--impl reference: the CPU implementation of the path on the host cores, at the full config (rank 0 only)."""
     if rank != 0:
         return
-    times, threads, t_ctor = port_sweeps(N_SAMPLES, N_LAYERS, args.warmup, args.steps)
+    times, threads, t_ctor = port_sweeps(N_SAMPLES, N_LAYERS, args.warmup, args.steps, dump=args.dump_outputs)
     total = float(np.sum(times))
     value = args.steps / total
     calib = None if args.no_calibration else reference_calibration()
@@ -475,6 +504,8 @@ def run_gpu(args, rank, world, local_rank):
     l0 = eng.launch_count()
     step_ms = timed_sweeps(eng, args.steps, flush, barrier, max_over_ranks, torch)
     launches = eng.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, engine_outputs(eng))     # before the e2e loops sweep the model further
     total_s = sum(step_ms) / 1e3
     value = (world if multi else 1) * args.steps / total_s
 
@@ -608,7 +639,11 @@ def main():
     ap.add_argument('--no-extras', action='store_true')
     ap.add_argument('--no-calibration', action='store_true')
     ap.add_argument('--config5-series', type=int, default=4096, help='series of the config-5 extra (BASELINE: 4096; fi mode runs on 1024 of them)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed to DIR/<name>.npy (float64); '
+                                                          'the inputs are seeded, so two builds can be compared file by file')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
