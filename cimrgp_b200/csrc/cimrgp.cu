@@ -1471,6 +1471,16 @@ int mrgp_create(const mrgp_config *cfg, const int64_t *const *region_offsets, co
     if (cfg->n_samples < 1) return fail(h, MRGP_EINVAL, "n_samples < 1");
     if (cfg->sample_begin < 0 || cfg->sample_end < cfg->sample_begin || cfg->sample_end > cfg->n_samples)
         return fail(h, MRGP_EINVAL, "bad sample range");
+    // the cluster size of the fused sweep must be a power of two the launch supports (0: chosen by the regions);
+    // anything else would only fail at the first sweep, far from its cause
+    int chain_cluster = 0;
+    if (const char *e = getenv("MRGP_CHAIN_CLUSTER")) {
+        char *end = nullptr;
+        const long c = strtol(e, &end, 10);
+        if (end == e || *end != '\0' || c < 0 || c > kChainMaxCluster || (c & (c - 1)))
+            return fail(h, MRGP_EINVAL, "MRGP_CHAIN_CLUSTER=\"%s\": must be 0 (by the regions), 1, 2, 4, 8 or %d", e, kChainMaxCluster);
+        chain_cluster = (int)c;
+    }
     h = new mrgp_handle();
     h->cfg = *cfg;
     if (const char *e = getenv("MRGP_OMEGA_BLOCK")) h->omega_warp = !(e[0] == '1');
@@ -1482,7 +1492,7 @@ int mrgp_create(const mrgp_config *cfg, const int64_t *const *region_offsets, co
     if (const char *e = getenv("MRGP_SPLIT")) h->split_kernels = !(e[0] == '0');
     if (const char *e = getenv("MRGP_CHAIN_PROF")) h->chain_prof_on = e[0] == '1';
     if (const char *e = getenv("MRGP_CHAIN_GUARD")) h->chain_guard_threshold = atof(e);
-    if (const char *e = getenv("MRGP_CHAIN_CLUSTER")) h->chain_cluster = atoi(e);
+    h->chain_cluster = chain_cluster;
     h->sharded = cfg->sample_end > cfg->sample_begin;   // an explicit range selects the exchange-buffer path
     h->lo = h->sharded ? cfg->sample_begin : 0;
     h->hi = h->sharded ? cfg->sample_end : cfg->n_samples;

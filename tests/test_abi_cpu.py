@@ -138,6 +138,21 @@ def test_create_rejects_what_the_reference_rejects():
         lib.mrgp_destroy(h)
 
 
+def test_create_checks_the_cluster_size_switch(monkeypatch):
+    """MRGP_CHAIN_CLUSTER (DESIGN.md §5c) is refused at creation unless the fused sweep can launch it."""
+    off = O.uniform_offsets(4096, 5, 2)
+    for value in ('0', '1', '2', '4', '8', '16'):
+        monkeypatch.setenv('MRGP_CHAIN_CLUSTER', value)
+        lib, rc, h = _create(4096, off)
+        assert rc == 0, (value, lib.mrgp_last_error(None))
+        lib.mrgp_destroy(h)
+    for value in ('3', '6', '12', '17', '32', '-1', '-16', '', 'x', '4x', '2.0', '99999999999'):
+        monkeypatch.setenv('MRGP_CHAIN_CLUSTER', value)
+        lib, rc, h = _create(4096, off)
+        assert rc == _lib.EINVAL and not h.value, value
+        assert b'MRGP_CHAIN_CLUSTER' in lib.mrgp_last_error(None), value
+
+
 def test_no_gpu_means_no_compute():
     import torch
     if torch.cuda.is_available():
