@@ -365,7 +365,10 @@ class MultiResolutionGaussianProcess(object):
         if index_set_obj is None:
             return self._engine.predict_var(self._warp(test_x))
         # MRGP.py:863-932.  The reference walks every layer of the MODEL with the test index set and overwrites the
-        # model's latent functions on the way; here the state is left untouched.
+        # model's latent functions on the way; here the state is left untouched.  A test region may be empty (fewer test
+        # points than regions): it holds no point whose moment it could change, so only the regions that hold test
+        # points are summed.  (The reference adds the latent variance at a region's first test point, :929, and cannot
+        # index the first point of an empty region.)
         test_offsets = offsets_of(index_set_obj)
         if len(test_offsets) != self.n_layers:
             raise ValueError('the test index set must have the resolutions of the training index set')

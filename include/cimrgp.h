@@ -244,7 +244,8 @@ int mrgp_predict_var(mrgp_handle *h, const double *x_test_dev, int64_t n_test, d
 /* Index-set form of the second moment (MRGP.py:863-932): sum over ALL layers of sum_i cm2_i phi_i^2 + bias_var +
  * n_test(region) / noise_mean + the latent variance of the region's first test point (MRGP.py:929).  The reference
  * overwrites the model's latent functions with their values at the test points while doing so (MRGP.py:893-901);
- * here they are derived quantities and the model state is left untouched.  out_dev (n_test,).               */
+ * here they are derived quantities and the model state is left untouched.  Test regions may be empty: a point takes
+ * the terms of the non-empty region that holds it in every layer.  out_dev (n_test,).                        */
 int mrgp_predict_var_indexed(mrgp_handle *h, const double *x_test_dev, int64_t n_test,
                              const int64_t *const *test_offsets, int32_t n_test_layers, double *out_dev);
 

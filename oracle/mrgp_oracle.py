@@ -702,6 +702,41 @@ class OracleMRGP(object):
         phi = eigenfunctions(xt, np.tile(ly.L[0], (xt.shape[0], 1)), self.M)
         return (phi ** 2) @ ly.cm2[0] + ly.bias_var[0]
 
+    def predict_var_indexed(self, test_x, test_offsets):
+        """MRGP.py:863-932 (index-set form of the second moment): per test point the sum over ALL layers j of
+        sum_i phi_i^2 cm2_i + bias_var + n_test(region) / noise_mean + f_var_j(first test point of the region), where
+        f_var_j is the latent variance of the layers < j (Stats.py:126-157) and the reference adds its value at the
+        region's FIRST test point, `latent_f_var[l][0]`, to every point of the region (:929).  Test points are assigned
+        to regions by position.  A region without test points contributes nothing (the reference cannot index its
+        first point); every point lies in a non-empty region, so the result is defined for every point."""
+        xt = self._norm_test(test_x)
+        if len(test_offsets) != self.J:
+            raise ValueError('the test index set must have the resolutions of the training index set')
+        n = xt.shape[0]
+        out = np.zeros(n)
+        fvar = np.zeros(n)   # latent variance of the layers below the current one, per test point
+        for j, off in enumerate(test_offsets):
+            ly = self.layers[j]
+            off = np.asarray(off, dtype=np.int64)
+            cnt = np.diff(off)
+            phi = eigenfunctions(xt, seg_expand(ly.L, off), self.M)
+            contrib = np.sum((phi ** 2) * seg_expand(ly.cm2, off), axis=1) + seg_expand(ly.bias_var, off)
+            first = np.zeros(ly.R)
+            full = cnt > 0
+            first[full] = fvar[off[:-1][full]]
+            out += contrib + seg_expand(cnt / ly.noise_mean + first, off)
+            fvar = fvar + contrib
+        return out
+
+    def test_likelihood(self, test, test_offsets=None):
+        """MRGP.py:825-831: mean over the test points of the Gaussian log density of ||y - mean|| with variance var
+        (index-set forms of both when test_offsets is given)."""
+        test_x, test_y = test[0], np.asarray(test[1], dtype=np.float64)
+        mf = self.predict_mean(test_x, test_offsets)
+        vf = self.predict_var(test_x) if test_offsets is None else self.predict_var_indexed(test_x, test_offsets)
+        ll = -0.5 * np.log(2 * np.pi * vf) - 0.5 * (la.norm(test_y - mf, axis=1) ** 2) / vf
+        return float(np.mean(ll))
+
     # ------------------------------------------------------------------------------------------
     def state(self):
         """Flat dict of every state array, the comparison surface for parity tests."""
