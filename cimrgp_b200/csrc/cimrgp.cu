@@ -2440,6 +2440,18 @@ int mrgp_elbo_wait(mrgp_handle *h, int32_t slot) {
     return MRGP_OK;
 }
 
+// Test offsets of one layer: cnt entries from 0 to n_test, non-decreasing (a test region may be empty).  The region
+// search of the prediction kernels assumes this order; decreasing offsets would put points in the wrong regions and
+// give k_eval_var_indexed a negative region count.
+static int check_test_offsets(mrgp_handle *h, const int64_t *off, size_t cnt, int64_t n_test, int j) {
+    if (off[0] != 0 || off[cnt - 1] != n_test) return fail(h, MRGP_EINVAL, "test offsets of layer %d do not cover the test points", j);
+    for (size_t r = 0; r + 1 < cnt; ++r)
+        if (off[r + 1] < off[r])
+            return fail(h, MRGP_EINVAL, "test offsets of layer %d must be non-decreasing (offset %zu: %lld < %lld)", j, r + 1,
+                        (long long)off[r + 1], (long long)off[r]);
+    return MRGP_OK;
+}
+
 int mrgp_predict_mean(mrgp_handle *h, const double *x_test_dev, int64_t n_test, const int64_t *const *test_offsets,
                       int32_t n_test_layers, double *out_dev) {
     int rc = check_ready(h, 0, true);
@@ -2455,7 +2467,7 @@ int mrgp_predict_mean(mrgp_handle *h, const double *x_test_dev, int64_t n_test, 
         size_t o = 0;
         for (int j = 0; j < n_test_layers; ++j) {
             const size_t cnt = h->plan[j].R + 1;
-            if (test_offsets[j][0] != 0 || test_offsets[j][cnt - 1] != n_test) return fail(h, MRGP_EINVAL, "test offsets of layer %d do not cover the test points", j);
+            if ((rc = check_test_offsets(h, test_offsets[j], cnt, n_test, j))) return rc;
             CK(cudaMemcpyAsync(staging + o, test_offsets[j], cnt * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
             dev_off.push_back(staging + o);
             o += cnt;
@@ -2489,7 +2501,7 @@ int mrgp_predict_var_indexed(mrgp_handle *h, const double *x_test_dev, int64_t n
     size_t o = 0;
     for (int j = 0; j < n_test_layers; ++j) {
         const size_t cnt = h->plan[j].R + 1;
-        if (test_offsets[j][0] != 0 || test_offsets[j][cnt - 1] != n_test) return fail(h, MRGP_EINVAL, "test offsets of layer %d do not cover the test points", j);
+        if ((rc = check_test_offsets(h, test_offsets[j], cnt, n_test, j))) return rc;
         CK(cudaMemcpyAsync(h->off_staging + o, test_offsets[j], cnt * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
         dev_off.push_back(h->off_staging + o);
         o += cnt;

@@ -236,7 +236,11 @@ int mrgp_elbo_wait(mrgp_handle *h, int32_t slot);
 
 /* x_test_dev (n_test, dx) normalised.  test_offsets == NULL: layer 0 / region 0 only (MRGP.py:726-755);
  * else test_offsets[j] (host, n_regions[j]+1 int64) assigns test points to regions by position for
- * the first n_test_layers layers (MRGP.py:757-803).  out_dev (n_test, dy).                          */
+ * the first n_test_layers layers (MRGP.py:757-803).  out_dev (n_test, dy).
+ * Test offsets of every layer run from 0 to n_test and must be non-decreasing; a region may be empty (equal
+ * neighbouring offsets).  Otherwise, as for n_test < 1 or n_test_layers outside [1, n_layers], MRGP_EINVAL with a
+ * message naming the layer.  The same holds for mrgp_predict_var_indexed, which takes exactly n_layers layers.
+ * Prediction is valid for test points with |x| / (2 L) < 2^30 in every layer (the range of the basis evaluation).  */
 int mrgp_predict_mean(mrgp_handle *h, const double *x_test_dev, int64_t n_test,
                       const int64_t *const *test_offsets, int32_t n_test_layers, double *out_dev);
 /* Layer-0 central second moment sum_i cm2_i phi_i^2 + bias_var (MRGP.py:833-861). out_dev (n_test,). */

@@ -14,15 +14,11 @@ import numpy as np
 import pytest
 
 from oracle import mrgp_oracle as O
-from parity import compare, mismatch
+from parity import compare
 import workloads
+from mrgp_helpers import Oracle, dropin, engine, ragged
 
 pytestmark = pytest.mark.gpu
-
-RTOL = 1e-6
-# fields downstream of the chain of permutation weights (see test_parity_gpu.py, OMEGA_CHAIN)
-OMEGA_CHAIN = ('S.B', 'S.kappa', 'S.logC', 'S.rho', 'S.omega')
-
 
 # ---- restated dispatch rules (the source of each is named; the tests assert the observable side of each) ------------
 def chain_solver_size(m):
@@ -55,32 +51,6 @@ def worker_tiers(r, n_w):
 
 
 # ---- helpers ----------------------------------------------------------------------------------------------------------
-def normed(x):
-    return (x - np.mean(x, 0)) / np.std(x, 0)     # the oracle's standard normalisation (MRGP.py:278-295)
-
-
-def ragged(n, counts, seed, min_len=3):
-    """Random region boundaries per layer (not nested across layers), every region at least min_len samples."""
-    rng = np.random.RandomState(seed)
-    out = []
-    for r in counts:
-        extra = rng.multinomial(n - min_len * r, rng.dirichlet(np.ones(r)))
-        out.append(np.r_[0, np.cumsum(min_len + extra)].astype(np.int64))
-    return out
-
-
-def engine(x, y, offsets, m, mode='ci', **kw):
-    from cimrgp_b200.engine import Engine
-    return Engine(normed(x), y, offsets, m, mode=mode, **kw)
-
-
-def dropin(x, y, m, resolution, fi, **kw):
-    from cimrgp_b200 import IndexSetUniform, LaplacianEigenpairs, MaternKernel
-    from cimrgp_b200.MRGP import MultiResolutionGaussianProcess
-    return MultiResolutionGaussianProcess([x, y], m, IndexSetUniform(x.shape[0], resolution, 2), LaplacianEigenpairs(),
-                                          MaternKernel(1, 1, 1), forced_independence=fi, **kw)
-
-
 def sweep(eng, k):
     eng.sweep(k)
     eng.synchronize()
@@ -107,110 +77,6 @@ def per_cta_samples(eng, layer=0):
     seg = np.zeros((n_seg.value, 6), dtype=np.int64)
     assert lib.mrgp_plan_segments(eng.handle, layer, seg.ctypes.data_as(C.POINTER(C.c_int64))) == 0
     return np.bincount(seg[:, 5], weights=seg[:, 1] - seg[:, 0], minlength=n_ctas.value).astype(np.int64)
-
-
-def omega_exact(lw, tol=1e-15):
-    """The doubly-stochastic scaling diag(e^a) exp(lw) diag(e^b) to roundoff: Newton's method on (a, b) with
-    backtracking, from 50 Sinkhorn sweeps.  On the nearly decomposable tables of models with many small regions over
-    many layers (log omega_hat spanning 1000 and more) plain Sinkhorn (mrgp_oracle.omega_sinkhorn) stops after its 10000
-    sweeps at column sums 1e-4 off; Newton converges quadratically there, to column sums within 1e-13 of one."""
-    from scipy.special import logsumexp
-    lw = np.asarray(lw, dtype=np.float64)
-    m = lw.shape[0]
-    la, lb = np.zeros(m), np.zeros(m)
-    for _ in range(50):
-        la = -logsumexp(lw + lb[None, :], axis=1)
-        lb = -logsumexp(lw + la[:, None], axis=0)
-
-    def resid(la, lb):
-        p = np.exp(lw + la[:, None] + lb[None, :])
-        return p, np.r_[p.sum(1) - 1, p.sum(0) - 1]
-
-    p, f = resid(la, lb)
-    for _ in range(100):
-        nf = np.max(np.abs(f))
-        if nf < tol:
-            break
-        jac = np.block([[np.diag(p.sum(1)), p], [p.T, np.diag(p.sum(0))]])
-        step = np.linalg.lstsq(jac, -f, rcond=None)[0]
-        t = 1.0
-        while t > 1e-6:
-            p2, f2 = resid(la + t * step[:m], lb + t * step[m:])
-            if np.max(np.abs(f2)) < nf:
-                break
-            t *= 0.5
-        else:
-            break
-        la, lb, p, f = la + t * step[:m], lb + t * step[m:], p2, f2
-    return p
-
-
-class Oracle(object):
-    """The NumPy oracle beside a device model.  In ci mode the reference solves for omega with MINPACK hybrd at xtol
-    1.5e-8 (Stats.py:413) while the device computes the exact doubly-stochastic scaling.  On some models hybrd stalls
-    ("not making good progress") and its slack in the omega chain exceeds the 1e-6 of the rule; every field downstream of
-    omega (ARD means, scale precisions, the coefficients of every layer after the next sweep) inherits it.  There, and
-    only after checking that the slack is the oracle's own (its omega chain differs from the exact scaling by more than
-    1e-6), the model is held to the same oracle with the exact scaling (omega_exact): every array at the rule, the shared
-    state at 1e-9, as test_config4_full_size_against_oracle does."""
-
-    def __init__(self, x, y, m, offsets, mode='ci', **kw):
-        self.args, self.kw = (x, y, m, offsets), dict(kw, mode=mode)
-        self.ora = O.OracleMRGP(x, y, m, offsets, **self.kw)
-        self.best = self.ora
-        self.exact = None
-        self.done = 0
-
-    def _sweep_exact(self, k):
-        saved = O.omega_sinkhorn
-        O.omega_sinkhorn = lambda lw: omega_exact(lw)
-        try:
-            for _ in range(k):
-                self.exact.sweep()
-        finally:
-            O.omega_sinkhorn = saved
-
-    def sweep(self, k):
-        for _ in range(k):
-            self.ora.sweep()
-        if self.exact is not None:
-            self._sweep_exact(k)
-        self.done += k
-
-    def check(self, eng):
-        got, ref = eng.state(), self.ora.state()
-        self.best = self.ora
-        try:
-            compare(got, ref)
-            return
-        except AssertionError:
-            if self.ora.mode == 'fi':
-                raise
-        if self.exact is None:
-            self.exact = O.OracleMRGP(*self.args, omega_solver='sinkhorn', **self.kw)
-            self._sweep_exact(self.done)
-        ex = self.exact.state()
-        assert any(mismatch(ref[k], ex[k], RTOL) is not None for k in OMEGA_CHAIN), \
-            'device off the oracle where the oracle agrees with its exact-scaling form'
-        self.best = self.exact
-        compare(got, ex)
-        for k in [k for k in ex if k.startswith('S.')]:
-            assert mismatch(got[k], ex[k], 1e-9, atol_scale=1e-9 if k == 'S.omega' else 1e-12) is None, k
-
-    def check_elbo(self, eng):
-        assert mismatch(eng.elbo(), self.best.elbo()[2], RTOL) is None
-
-    def check_predictions(self, eng, n_test=2000, seed=11):
-        """predict_mean without and with an index set (every layer), predict_var."""
-        ora = self.best
-        counts = [len(o) - 1 for o in self.args[3]]
-        n_test = max(n_test, 4 * max(counts))
-        xt = np.atleast_2d(np.linspace(1, 3, n_test)).T
-        xtn = (xt - ora.mean_x) / ora.std_x
-        toff = ragged(n_test, counts, seed, min_len=1)
-        assert mismatch(eng.predict_mean(xtn), ora.predict_mean(xt), RTOL) is None
-        assert mismatch(eng.predict_mean(xtn, toff), ora.predict_mean(xt, toff), RTOL) is None
-        assert mismatch(eng.predict_var(xtn), ora.predict_var(xt), RTOL) is None
 
 
 def run_against_oracle(eng, ora, elbo=True, predict=True):

@@ -8,6 +8,7 @@ import pytest
 
 from oracle import mrgp_oracle as O
 from parity import mismatch
+from mrgp_helpers import prediction_ld, ragged, with_empty_regions
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 RTOL = 1e-9
@@ -65,26 +66,6 @@ def _loop_moments(m, xt, toff):
     return mean, var
 
 
-def with_empty_regions(n_test, counts, seed):
-    """Test offsets per layer with the given region counts; the first and last region of every layer with more than
-    two regions are empty, and so is a run of three in the middle when there are more than eight.  With fewer test
-    points than the remaining regions, a random choice of them holds one point each."""
-    rng = np.random.RandomState(seed)
-    out = []
-    for r in counts:
-        sizes = np.zeros(r, dtype=np.int64)
-        full = np.arange(r)
-        if r > 2:
-            full = full[1:-1]
-        if r > 8:
-            full = np.setdiff1d(full, np.arange(r // 2 - 2, r // 2 + 1))
-        if n_test < len(full):
-            full = np.sort(rng.choice(full, n_test, replace=False))
-        sizes[full] = rng.multinomial(n_test - len(full), np.ones(len(full)) / len(full)) + 1
-        out.append(np.r_[0, np.cumsum(sizes)].astype(np.int64))
-    return out
-
-
 @pytest.mark.parametrize('mode', ['ci', 'fi'])
 def test_prediction_with_empty_test_regions(mode):
     """A test index set with fewer points than regions: the mean is the sum over layers at each point's own region,
@@ -116,3 +97,54 @@ def test_indexed_second_moment_needs_every_layer():
     _, m, res = fitted('predvar_ci')
     with pytest.raises(ValueError):
         m.predict_var_indexed(np.ones((10, 1)), O.uniform_offsets(10, res - 1, 2))
+
+
+def edge_test_sets(st, counts, x_lo, x_hi, seed):
+    """Normalised test points and test offsets at the edges of prediction: 1 to 129 points (across the 128-thread
+    block of the kernels) with empty first, last and middle regions and with ragged regions that may be empty, points in
+    random order with exact duplicates, and points exactly at -L, +L of every region of the last layer (each in that
+    region) and at x = 0.  Yields (name, x (n,), offsets)."""
+    rng = np.random.RandomState(seed)
+    for n_test in (1, 7, 40, 127, 128, 129):
+        x = rng.uniform(x_lo, x_hi, n_test)
+        yield 'empty%d' % n_test, x, with_empty_regions(n_test, counts, seed=n_test)
+        yield 'ragged%d' % n_test, x, ragged(n_test, counts, seed=n_test, min_len=0)
+    pool = rng.uniform(x_lo, x_hi, 37)
+    x = pool[rng.randint(0, 37, 500)]
+    assert len(np.unique(x)) < 500 and np.any(np.diff(x) < 0)
+    yield 'shuffled_duplicates', x, ragged(500, counts, seed=seed, min_len=0)
+    j = len(counts) - 1
+    L = st['L%d.L' % j][:, 0]
+    x = np.r_[np.stack([-L, L], axis=1).ravel(), 0.0]
+    offs = ragged(x.shape[0], counts[:-1], seed=seed + 1, min_len=0)
+    last = np.r_[np.arange(counts[-1]) * 2, x.shape[0]].astype(np.int64)   # -L_r, +L_r in region r; 0 in the last
+    yield 'interval_edges', x, offs + [last]
+
+
+@pytest.mark.parametrize('mode', ['ci', 'fi'])
+def test_long_double_prediction_matches_oracle(mode):
+    """The long-double restatement of prediction (mrgp_helpers.prediction_ld), which the device tests use as the
+    reference of the evaluation kernels, against the oracle's predictions on the oracle's own fitted state, at 1e-12:
+    global and index-set mean and second moment, on the edge sets of the device tests (empty regions included)."""
+    g = np.load(os.path.join(GOLD, 'c1_ci.npz'))
+    res = int(g['meta.resolution'])
+    m = O.OracleMRGP(g['x'], g['y'], 30, O.uniform_offsets(g['x'].shape[0], res, 2), mode=mode)
+    for _ in range(3):
+        m.sweep()
+    st = m.state()
+    counts = [2 ** j for j in range(res + 1)]
+    raw = lambda xn: xn[:, None] * m.std_x + m.mean_x
+    seen_empty = False
+    for name, xn, toff in edge_test_sets(st, counts, -1.5, 1.5, seed=5):
+        xt = raw(xn)
+        xn = m._norm_test(xt)[:, 0]          # the oracle normalises again: use its points
+        seen_empty |= any(np.any(np.diff(o) == 0) for o in toff)
+        mean, _, var, _ = prediction_ld(st, xn, m.M)
+        assert mismatch(mean, m.predict_mean(xt), 1e-12) is None, name
+        assert mismatch(var, m.predict_var(xt), 1e-12) is None, name
+        mean, _, var, _ = prediction_ld(st, xn, m.M, toff)
+        assert mismatch(mean, m.predict_mean(xt, toff), 1e-12) is None, name
+        assert mismatch(var, m.predict_var_indexed(xt, toff), 1e-12) is None, name
+        mean, _, var, _ = prediction_ld(st, xn, m.M, toff[:2])
+        assert var is None and mismatch(mean, m.predict_mean(xt, toff[:2]), 1e-12) is None, name
+    assert seen_empty
