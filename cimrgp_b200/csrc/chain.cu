@@ -1020,19 +1020,10 @@ __global__ void __launch_bounds__(kChainThreads, 1) k_ci_sweep(const ChainModel 
 
     // ---- prologue: the small-matrix state into L2 (the sweep is a chain of dependent loads), omega (transposed) and the
     //      warm starts on CTA 0, the ARD mean of the previous sweep everywhere ---------------------------------------
-    if (C >= 4 && rank >= 2 && m.pf_mode != 0) {   // CTAs that are neither on the chain (0) nor own layer 0's region (1) pull the state into L2
+    if (C >= 4 && rank >= 2) {   // CTAs that are neither on the chain (0) nor own layer 0's region (1) pull the state into L2
         const unsigned long long lines = m.pf_lines, nthr = (unsigned long long)(C - 2) * kChainThreads;
         const unsigned long long first = (unsigned long long)(rank - 2) * kChainThreads + tid;
-        if (m.pf_mode == 2) {    // bulk prefetches (the TMA unit walks the lines): 4 KB per instruction
-            constexpr unsigned long long kChunk = 4096;
-            const unsigned long long bytes = lines * 128;
-            for (unsigned long long off = first * kChunk; off < bytes; off += nthr * kChunk) {
-                const unsigned sz = (unsigned)(bytes - off < kChunk ? bytes - off : kChunk);
-                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(m.pf_base + off), "r"(sz) : "memory");
-            }
-        } else {
-            for (unsigned long long l = first; l < lines; l += nthr) asm volatile("prefetch.global.L2 [%0];" ::"l"(m.pf_base + l * 128));
-        }
+        for (unsigned long long l = first; l < lines; l += nthr) asm volatile("prefetch.global.L2 [%0];" ::"l"(m.pf_base + l * 128));
     }
     if (rank == 0) {
         for (int t = tid; t < M * M; t += kChainThreads) {

@@ -144,14 +144,11 @@ struct mrgp_handle {
     bool chain_uploaded = false;     // the device descriptor matches the current pointers (reset by drop_graph)
     uint64_t generation = 0;         // bumped whenever a captured sweep / descriptor becomes stale (groups re-capture)
     uint64_t stream_ops = 0;         // asynchronous work queued on the handle's stream from outside a sweep (groups order after it)
-    bool split_kernels = false;      // MRGP_SPLIT=1: lane-split statistics kernel (experiment, 30 % slower: profiles/r02_ncu_summary.md)
     bool fused = true;               // MRGP_FUSED=0: the multi-kernel sweep of round 1
-    int chain_pf_mode = 1;           // MRGP_CHAIN_PF: L2 prefetch of the state by the fused sweep (0 off, 1 per line, 2 bulk)
-    bool direct_launch = false;      // MRGP_DIRECT=1: the fused sweep is launched on the stream, not through a graph (experiment)
-    bool skip_l0_fallback = false;   // MRGP_NO_L0_FALLBACK=1: timing experiment only (the guard still reports)
+    bool direct_launch = false;      // the fused sweep is launched on the stream, not through a graph (set once prefetched
+                                     // observations are taken over: the buffers alternate, a graph would hold one pointer)
     int chain_cluster = 0;           // CTAs per model of the fused sweep (0: by the number of regions)
     bool inferred_shortcut = true;   // skip phase A where Phi^T r == 0 identically (MRGP_STREAM_ALL=1: stream everything)
-    bool omega_warp = true;   // single-warp register-resident omega solve for M <= 32 (MRGP_OMEGA_BLOCK=1: block version)
     // peer-memory exchange (multi-GPU): arena + flags in one cudaMalloc'ed block that the peers map through CUDA IPC
     struct Comm {
         bool exported = false, ready = false;
@@ -820,13 +817,13 @@ int do_mid_ci(mrgp_handle *h, int j, bool fork_omega, bool zero_T) {
             k_ard<<<1, kOmegaThreads, smem, st>>>(a, n_partials);
             CK(cudaGetLastError());
         }
-        if (h->omega_warp && M == 30) {
+        if (M == 30) {
             CK(cudaFuncSetAttribute(k_scale_warp<30>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
             k_scale_warp<30><<<1, 64, 0, st>>>(a);
-        } else if (h->omega_warp && M == 20) {
+        } else if (M == 20) {
             CK(cudaFuncSetAttribute(k_scale_warp<20>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
             k_scale_warp<20><<<1, 64, 0, st>>>(a);
-        } else if (h->omega_warp && M == 8) {
+        } else if (M == 8) {
             CK(cudaFuncSetAttribute(k_scale_warp<8>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
             k_scale_warp<8><<<1, 64, 0, st>>>(a);
         } else {
@@ -1101,13 +1098,6 @@ int do_exchange(mrgp_handle *h, int j, int slot, int nv, bool is_max);
 template <int M>
 cudaError_t launch_ystats(mrgp_handle *h, const StreamArgs &a) {
     constexpr int DY = 2;
-    if (h->split_kernels) {   // lane-split form: 512 threads, DY lanes per sample
-        const size_t smem2 = (size_t)(kStages * TileLayout<DY, true, false, false>::kDoubles) * sizeof(double);
-        cudaError_t e2 = set_smem(k_ystats_split<DY, M>, smem2);
-        if (e2 != cudaSuccess) return e2;
-        k_ystats_split<DY, M><<<h->n_ctas, kThreadsS, smem2, h->stream>>>(a);
-        return cudaGetLastError();
-    }
     const size_t smem = (size_t)(kStages * TileLayout<DY, true, false, false>::kDoubles + kRedSmemDoubles) * sizeof(double);
     cudaError_t e = set_smem(k_ystats<DY, M>, smem);
     if (e != cudaSuccess) return e;
@@ -1141,7 +1131,7 @@ int do_ystats(mrgp_handle *h) {
     StreamArgs a = stream_args(h, 0);
     // one handle: the last CTA of the pass sums the run partials itself (no second launch); sharded: the partials of
     // the ranks' chunks are exchanged first
-    const bool fuse = !h->sharded && !h->split_kernels && lp.R <= 64;
+    const bool fuse = !h->sharded && lp.R <= 64;
     a.fuse_tail = fuse ? 1 : 0;
     a.yc_out = d.yc;
     a.ysum_out = d.ysum;
@@ -1181,7 +1171,6 @@ int upload_chain_model(mrgp_handle *h) {
     m.J = h->cfg.n_layers;
     m.M = h->cfg.n_basis;
     m.DY = h->cfg.dy;
-    m.pf_mode = h->chain_pf_mode;
     m.sbase = reinterpret_cast<double *>(h->ws + h->state_begin);
     m.pf_base = h->ws + h->state_begin;
     m.pf_lines = (h->state_end - h->state_begin + 127) / 128;
@@ -1236,7 +1225,7 @@ int do_fused_sweep(mrgp_handle *h) {
     // terms; when the residual is tiny against sum |y|^2 (ratio below kChainGuard: high-SNR data) the sweep sets the
     // model's status word and the kernel below - a no-op otherwise - takes the statistics of layer 0 by a pass over the
     // samples and repeats its bias / noise update (nothing else of the sweep depends on them).
-    if (h->sharded || h->skip_l0_fallback) return MRGP_OK;   // (the sharded handle reports the status; its fallback would need an exchange)
+    if (h->sharded) return MRGP_OK;   // (the sharded handle reports the status; its fallback would need an exchange)
     if (ystats_small(h)) {
         const int e = launch_l0_fix_small(chain_solver_size(h->cfg.n_basis), h->chain_ptr_dev, 1, h->plan[0].R, h->stream);
         if (e != 0) return fail(h, MRGP_ECUDA, "layer-0 fallback launch: %s", cudaGetErrorString((cudaError_t)e));
@@ -1349,11 +1338,9 @@ FieldRef field_ref(mrgp_handle *h, int layer, int field) {
         if (layer != -1) return f;
         SharedDev &s = h->sh;
         switch (field) {
-            case 54: f = {h->chain_prof, (int64_t)h->cfg.n_layers * 16}; break;
+            case 54: f = {h->chain_prof, (int64_t)h->cfg.n_layers * 16}; break;   // MRGP_CHAIN_PROF=1: clock stamps of the fused sweep
             case 56: f = {h->chain_tables, (int64_t)h->cfg.n_layers * h->cfg.n_basis * h->cfg.n_basis}; break;   // (J, M, M) tables of the last sweep
-            case MRGP_F_FUSED_GUARD: f = {h->chain_guard, 2}; break;   // MRGP_CHAIN_PROF=1: clock stamps of the fused sweep
-            case 52: f = {s.omegaK + 64 * 64 + 32, 3}; break;
-            case 53: f = {s.omegaK + 64 * 64 + 40, 5}; break;   // MRGP_OMEGA_PROF builds: cycles of the k_ard phases   // MRGP_OMEGA_PROF builds: cycles of the Newton stages
+            case MRGP_F_FUSED_GUARD: f = {h->chain_guard, 2}; break;
             case MRGP_F_AXIS_B: f = {s.axB, (int64_t)M * DY * DY}; break;
             case MRGP_F_AXIS_KAPPA: f = {s.axKappa, (int64_t)M * DY}; break;
             case MRGP_F_AXIS_RHO: f = {s.axRho, (int64_t)M * DY}; break;
@@ -1483,13 +1470,8 @@ int mrgp_create(const mrgp_config *cfg, const int64_t *const *region_offsets, co
     }
     h = new mrgp_handle();
     h->cfg = *cfg;
-    if (const char *e = getenv("MRGP_OMEGA_BLOCK")) h->omega_warp = !(e[0] == '1');
     if (const char *e = getenv("MRGP_STREAM_ALL")) h->inferred_shortcut = !(e[0] == '1');
     if (const char *e = getenv("MRGP_FUSED")) h->fused = !(e[0] == '0');
-    if (const char *e = getenv("MRGP_CHAIN_PF")) h->chain_pf_mode = atoi(e);
-    if (const char *e = getenv("MRGP_DIRECT")) h->direct_launch = e[0] == '1';
-    if (const char *e = getenv("MRGP_NO_L0_FALLBACK")) h->skip_l0_fallback = e[0] == '1';
-    if (const char *e = getenv("MRGP_SPLIT")) h->split_kernels = !(e[0] == '0');
     if (const char *e = getenv("MRGP_CHAIN_PROF")) h->chain_prof_on = e[0] == '1';
     if (const char *e = getenv("MRGP_CHAIN_GUARD")) h->chain_guard_threshold = atof(e);
     h->chain_cluster = chain_cluster;
@@ -1747,17 +1729,15 @@ int mrgp_set_observations(mrgp_handle *h, const double *y_dev) {
     return MRGP_OK;
 }
 
-// Host-to-device copy in pieces of MRGP_H2D_CHUNK_MB (default 4, 0: one copy).  In isolation 16 MB from pinned memory took
-// 0.47 ms as one cudaMemcpyAsync and 0.31 ms as 4 MB pieces on the boxes of this project (scratch/h2d_bw.py, noisy); inside
-// bench.py the piece size made no difference (the copy is hidden behind the sweep).
+// Host-to-device copy in pieces of kH2DChunk bytes.  In isolation 16 MB from pinned memory took 0.47 ms as one
+// cudaMemcpyAsync and 0.31 ms as 4 MB pieces on the boxes of this project (scratch/h2d_bw.py, noisy); inside bench.py the
+// piece size made no difference (the copy is hidden behind the sweep).
+constexpr size_t kH2DChunk = (size_t)4 << 20;
+
 static cudaError_t copy_h2d_chunked(void *dst, const void *src, size_t bytes, cudaStream_t st) {
-    static const size_t chunk = [] {
-        const char *e = getenv("MRGP_H2D_CHUNK_MB");
-        return (size_t)(e ? atoi(e) : 4) << 20;
-    }();
-    if (chunk == 0 || bytes <= chunk) return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
-    for (size_t off = 0; off < bytes; off += chunk) {
-        const size_t n = bytes - off < chunk ? bytes - off : chunk;
+    if (bytes <= kH2DChunk) return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
+    for (size_t off = 0; off < bytes; off += kH2DChunk) {
+        const size_t n = bytes - off < kH2DChunk ? bytes - off : kH2DChunk;
         cudaError_t e = cudaMemcpyAsync(static_cast<char *>(dst) + off, static_cast<const char *>(src) + off, n, cudaMemcpyHostToDevice, st);
         if (e != cudaSuccess) return e;
     }

@@ -46,7 +46,7 @@ struct ChainLayer {
 };
 
 struct ChainModel {
-    int32_t J, M, DY, pf_mode;     // pf_mode: L2 prefetch of the state at the start of a sweep (0 off, 1 per line, 2 bulk)
+    int32_t J, M, DY;
     double *sbase;                 // base of the small-matrix state in the workspace (AncEntry offsets are relative to it)
     const char *pf_base;           // range pulled into L2 at the start of a sweep (the small-matrix state), 128-byte lines
     unsigned long long pf_lines;

@@ -666,161 +666,6 @@ __global__ void __launch_bounds__(kThreads, 1) k_ystats(StreamArgs p) {
     }
 }
 
-// ------------------------------------------------------------------------------------------------
-// Lane-split form of the streaming kernels: DY lanes per sample, every lane owns ONE output dimension of the sample
-// (its column of Phi^T y / Phi^T r, its residual) and repeats the basis recurrence.  A thread then carries M + 2
-// accumulators instead of DY M + 3: half the registers, 512-thread CTAs (16 warps per SM instead of 8), and the
-// dependent FMAs of an accumulator are far enough apart for the FP64 pipe.  Price: the seed and the recurrence are
-// computed DY times per sample.
-// ------------------------------------------------------------------------------------------------
-constexpr int kThreadsS = 512;
-
-// Sums over the threads of the block that own the same output dimension, fixed order: out index by (value, dim).
-template <int NV, int DY>
-__device__ __forceinline__ void block_reduce_split(const double (&v)[NV], double *sm /* [16][NV][DY] */, double (&res)[1], int &res_index) {
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    __syncthreads();
-#pragma unroll
-    for (int k = 0; k < NV; ++k) {
-        double t = v[k];
-#pragma unroll
-        for (int o = 16; o >= DY; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
-        if (lane < DY) sm[(warp * NV + k) * DY + lane] = t;
-    }
-    __syncthreads();
-    res_index = -1;
-    if (tid < NV * DY) {
-        double t = 0.0;
-#pragma unroll
-        for (int w = 0; w < kThreadsS / 32; ++w) t += sm[w * NV * DY + tid];
-        res[0] = t;
-        res_index = tid;      // = value * DY + dim
-    }
-}
-
-template <int DY, int M, int SB>
-__device__ __forceinline__ void ystats_split_block(double (&T)[M + 2], const double *st, int k0, int lo_rel, int hi_rel, double inv2L,
-                                                   double rs) {
-    using L = TileLayout<DY, true, false, false>;
-    const int pair = threadIdx.x / DY, d = threadIdx.x % DY;
-    double c2[SB], f[SB], fm[SB], yv[SB];
-#pragma unroll
-    for (int q = 0; q < SB; ++q) {
-        const int idx = (k0 + q) * kThreads + pair;
-        const bool act = idx >= lo_rel && idx < hi_rel;
-        const double x = act ? st[L::kX + idx] : 0.0;
-        basis_seed(x, inv2L, act ? rs : 0.0, f[q], c2[q]);
-        fm[q] = 0.0;
-        yv[q] = act ? st[L::kY + idx * DY + d] : 0.0;
-        T[M] += yv[q];
-        T[M + 1] = fma(yv[q], yv[q], T[M + 1]);
-    }
-#pragma unroll
-    for (int i = 0; i < M; ++i) {
-#pragma unroll
-        for (int q = 0; q < SB; ++q) {
-            T[i] = fma(f[q], yv[q], T[i]);
-            const double fn = fma(c2[q], f[q], -fm[q]);
-            fm[q] = f[q];
-            f[q] = fn;
-        }
-    }
-}
-
-template <int DY, int M>
-__global__ void __launch_bounds__(kThreadsS, 1) k_ystats_split(StreamArgs p) {
-    using L = TileLayout<DY, true, false, false>;
-    static_assert(kThreadsS / DY == kThreads, "a sub-block of the tile is kThreads samples");
-    constexpr int NCW = kThreadsS / 32, NV = M + 2;
-    extern __shared__ __align__(128) double dsm[];
-    double *stages = dsm;
-    __shared__ double red[NCW * NV * DY];
-    __shared__ __align__(8) uint64_t full_bar[kStages];
-    __shared__ __align__(8) uint64_t empty_bar[kStages];
-    const int tid = threadIdx.x, lane = tid & 31;
-    const int64_t c0 = p.sample_begin + (int64_t)blockIdx.x * p.cta_quantum;
-    const int64_t c1 = (c0 + p.cta_quantum < p.n_samples) ? c0 + p.cta_quantum : p.n_samples;
-    const int n_tiles = (c1 > c0) ? (int)((c1 - c0 + kTile - 1) / kTile) : 0;
-    if (tid == 0) {
-#pragma unroll
-        for (int s = 0; s < kStages; ++s) {
-            mbar_init(&full_bar[s], 1);
-            mbar_init(&empty_bar[s], NCW);
-        }
-        mbar_fence_init();
-    }
-    __syncthreads();
-    int next_issue = 0;
-    double T[NV];
-#pragma unroll
-    for (int i = 0; i < NV; ++i) T[i] = 0.0;
-    int s = p.cta_seg[blockIdx.x];
-    const int s_end = p.cta_seg[blockIdx.x + 1];
-    int loaded = -1;
-    double inv2L = 0.0, rs = 0.0;
-    Segment sg;
-    if (s < s_end) sg = p.segs[s];
-    for (int t = 0; t < n_tiles; ++t) {
-        const int stage = t % kStages;
-        const double *st = stages + stage * L::kDoubles;
-        if (tid == 0) refill<DY, true, false, false>(p, stages, full_bar, empty_bar, next_issue, t, n_tiles, c0, c1);
-        mbar_wait(&full_bar[stage], (uint32_t)((t / kStages) & 1));
-        const int64_t tile_lo = c0 + (int64_t)t * kTile;
-        const int64_t tile_hi = (tile_lo + kTile < c1) ? tile_lo + kTile : c1;
-        int64_t pos = tile_lo;
-        while (pos < tile_hi) {
-            if (loaded != s) {
-                inv2L = p.inv2L[sg.region];
-                rs = p.rsqrtL[sg.region];
-                loaded = s;
-            }
-            const int64_t seg_end = sg.start + sg.len;
-            const int64_t hi = (seg_end < tile_hi) ? seg_end : tile_hi;
-            int ka = (int)((pos - tile_lo) / kThreads);
-            const int kb = (int)((hi - 1 - tile_lo) / kThreads);
-            while (ka <= kb) {
-                const int left = kb - ka + 1;
-                if (left >= 3) {
-                    ystats_split_block<DY, M, 4>(T, st, ka, (int)(pos - tile_lo), (int)(hi - tile_lo), inv2L, rs);
-                    ka += 4;
-                } else if (left >= 2) {
-                    ystats_split_block<DY, M, 2>(T, st, ka, (int)(pos - tile_lo), (int)(hi - tile_lo), inv2L, rs);
-                    ka += 2;
-                } else {
-                    ystats_split_block<DY, M, 1>(T, st, ka, (int)(pos - tile_lo), (int)(hi - tile_lo), inv2L, rs);
-                    ka += 1;
-                }
-            }
-            pos = hi;
-            if (hi == seg_end) {
-                if (sg.flush) {
-                    // partial layout of k_ystats: [c (M*DY) | sum y (DY) | sum |y|^2]
-                    double res[1];
-                    int idx;
-                    block_reduce_split<NV, DY>(T, red, res, idx);
-                    double *out = p.part + (size_t)sg.run * p.part_stride;
-                    if (idx >= 0 && idx < (M + 1) * DY) out[idx] = res[0];          // c and sum y: index = value * DY + dim
-                    if (idx >= (M + 1) * DY) red[idx - (M + 1) * DY] = res[0];      // sum y_d^2 per dimension
-                    __syncthreads();
-                    if (tid == 0) {
-                        double t2 = 0.0;
-#pragma unroll
-                        for (int dd = 0; dd < DY; ++dd) t2 += red[dd];
-                        out[M * DY + DY] = t2;
-                    }
-                    __syncthreads();
-#pragma unroll
-                    for (int i = 0; i < NV; ++i) T[i] = 0.0;
-                }
-                ++s;
-                if (s < s_end) sg = p.segs[s];
-            }
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&empty_bar[stage]);
-    }
-}
-
 // yc[r][i][d], ysum[r][0..DY] = sums over the region's runs of the k_ystats partials (fixed order).
 // (MP: the padded number of basis functions the partials were written for.)  1024 threads: value = tid % 64 (chunks of
 // 64 values), 16 slices over the runs with their loads in flight together, combined in slice order.
@@ -1432,13 +1277,6 @@ __global__ void __launch_bounds__(kOmegaThreads) k_ard(RegionArgs a, int n_parti
     const int NVP = (3 * M + 31) & ~31, NVWP = (4 * M + 31) & ~31;
     double *s_data = s_part + NW * M, *s_half = s_data + NVP, *s_w = s_half + 2 * NVP;   // B sums, scratch, ARD sums
     ts_begin(a.ts, a.layer * 4 + 3);
-#ifdef MRGP_OMEGA_PROF
-    long long pc[6];
-    pc[0] = clock64();
-#define ARD_PC(k) pc[k] = clock64()
-#else
-#define ARD_PC(k)
-#endif
     // one wave of global loads: the per-CTA sums of k_mid1 (data part of B: same code as k_mid2, same bits; ARD sums:
     // one value per thread, k_mid1 runs at most 32 CTAs) go to registers while every other input is staged in
     // shared memory
@@ -1506,7 +1344,6 @@ __global__ void __launch_bounds__(kOmegaThreads) k_ard(RegionArgs a, int n_parti
         a.axCov[i * 4 + 3] = bg.cov[2];
         // sum_l m2_li / S_li = sum_l 1/(prec S) + tr((sum_l zeta^2 y y^T / S) C_i)
         const double beta2 = s_w[i * 4 + 0] + (s_w[i * 4 + 1] * bg.cov[0] + 2.0 * s_w[i * 4 + 2] * bg.cov[1] + s_w[i * 4 + 3] * bg.cov[2]);
-        ARD_PC(1);
         // ARD update of the same basis function in the same thread (no barrier: its sums do not depend on the axis
         // update and fill the latency of the chain above)
         double sh = 0.0, sc = 0.0;
@@ -1526,7 +1363,6 @@ __global__ void __launch_bounds__(kOmegaThreads) k_ard(RegionArgs a, int n_parti
         s_lmean[i] = lmean;
     }
     __syncthreads();
-    ARD_PC(2);
     for (int t = tid; t < M * M; t += kOmegaThreads) {
         const int i = t / M, k = t % M;
         const double *C = s_C + i * 4, *B = s_B + k * 4;
@@ -1540,7 +1376,6 @@ __global__ void __launch_bounds__(kOmegaThreads) k_ard(RegionArgs a, int n_parti
     // column shifts (row shifts cancel in the row normalisation).  One thread per row, then one per column: a serial
     // chain of M maxima is shorter than the rounds of warp reductions it replaces.
     __syncthreads();
-    ARD_PC(3);
     double *s_rowmax = s_part, *s_colmax = s_part + M;   // the partial sums are no longer needed
     if (tid < M) {
         double mx = -INFINITY;
@@ -1555,16 +1390,10 @@ __global__ void __launch_bounds__(kOmegaThreads) k_ard(RegionArgs a, int n_parti
         a.omegaK[64 * 64 + tid] = mx;
     }
     __syncthreads();
-    ARD_PC(4);
     for (int t = tid; t < M * M; t += kOmegaThreads) {
         const int k = t / M, i = t % M;        // column-major output: coalesced stores
         a.omegaK[t] = exp((P[i * M + k] - s_rowmax[i]) - s_colmax[k]);
     }
-    ARD_PC(5);
-#ifdef MRGP_OMEGA_PROF
-    if (tid == 0)
-        for (int k = 0; k < 5; ++k) a.omegaK[64 * 64 + 40 + k] = (double)(pc[k + 1] - pc[k]);
-#endif
     ts_dbg(a.ts, a.layer, 0, false);   // debug slots: [0] = (k_ard begin, k_ard end)
     ts_dbg(a.ts, a.layer, 0, true);
 }
@@ -1848,9 +1677,6 @@ __global__ void __launch_bounds__(64, 1) k_scale_warp(RegionArgs a) {
         }
         err_prev = err;
         last = kOmegaNewton;
-#ifdef MRGP_OMEGA_PROF
-        const long long pc0 = clock64();
-#endif
         // ---- Newton matrix: lane j builds row j of diag(c) - P^T P + 1/M from its column Q and the transposed table
         double H[M];
 #pragma unroll
@@ -1871,9 +1697,6 @@ __global__ void __launch_bounds__(64, 1) k_scale_warp(RegionArgs a) {
         }
         // ---- Cholesky (right-looking, lane = row) fused with the forward substitution; the next pivot is formed
         //      first in every step (one shuffle) so that its reciprocal square root overlaps the rank-1 update
-#ifdef MRGP_OMEGA_PROF
-        const long long pc1 = clock64();
-#endif
         double rhs = 1.0 - c, y = 0.0, dinv = 0.0;
         double piv = __shfl_sync(0xffffffffu, H[0], 0);
         double *colbuf = T;                                           // the transposed table is no longer needed
@@ -1896,9 +1719,6 @@ __global__ void __launch_bounds__(64, 1) k_scale_warp(RegionArgs a) {
 #pragma unroll
             for (int j = k + 1; j < M; ++j) H[j] = fma(-H[k], cb[j], H[j]);   // broadcast loads of l_jk
         }
-#ifdef MRGP_OMEGA_PROF
-        const long long pc2 = clock64();
-#endif
         // ---- L^T x = y with the transposed factor: lane i reads l_ki, k > i, from shared memory -------------------
         __syncwarp();
 #pragma unroll
@@ -1921,14 +1741,6 @@ __global__ void __launch_bounds__(64, 1) k_scale_warp(RegionArgs a) {
             if (lane < k) y = fma(-Q[k], xk, y);
         }
         if (row) v = fmax(1e-280, fmin(1e280, v * exp(fmax(-30.0, fmin(30.0, x)))));
-#ifdef MRGP_OMEGA_PROF
-        if (lane == 0) {
-            const long long pc3 = clock64();
-            a.omegaK[64 * 64 + 32 + 0] = (double)(pc1 - pc0);
-            a.omegaK[64 * 64 + 32 + 1] = (double)(pc2 - pc1);
-            a.omegaK[64 * 64 + 32 + 2] = (double)(pc3 - pc2);
-        }
-#endif
     }
     ts_dbg(a.ts, a.layer, 2, true);
     // last resort: plain Sinkhorn sweeps (see omega_solve_serial); on model tables the loop exits at its first test

@@ -132,13 +132,13 @@ def test_basis_size_edges_at_mid_size(m):
 
 @pytest.mark.parametrize('m', [24, 32])
 def test_multi_kernel_sweep_with_the_block_omega_solver(m, monkeypatch):
-    """MRGP_FUSED=0 MRGP_OMEGA_BLOCK=1: the multi-kernel sweep with the one-CTA omega solve for M <= 32."""
+    """MRGP_FUSED=0 at M = 24 and 32: the multi-kernel sweep takes the one-CTA omega solve (k_scale), because the
+    single-warp solver (k_scale_warp) is instantiated only for M = 8, 20 and 30."""
     n, resolution = 3000, 4
     x, y = workloads.workload1(n)
     offsets = O.uniform_offsets(n, resolution, 2)
     want = fused_launches(x, y, offsets)
     monkeypatch.setenv('MRGP_FUSED', '0')
-    monkeypatch.setenv('MRGP_OMEGA_BLOCK', '1')
     eng = engine(x, y, offsets, m)
     run_against_oracle(eng, Oracle(x, y, m, offsets))
     assert launches_per_sweep(eng) > want
