@@ -230,6 +230,12 @@ __device__ __forceinline__ void mid1_layer0(const ChainModel &m, const ChainLaye
     if (on) p1_finish(ly, ri, t0, t1, dsum, S, noise, ardMean[lane], acc);
 }
 
+// Regions a worker warp takes at once in P1-finish / in S2 + P4 / P5 of the layers above the first: ONE form per step,
+// whatever the number of regions (unused slots are masked), so that its code is fetched once, at the first layer, and
+// not for the first time on the fine layers after an L2 flush.  Layer 9 at config 4 (512 regions on 120 worker warps)
+// is one batch of each.
+constexpr int kMid1Batch = 8, kFinishBatch = 5;
+
 // Layers above the first (targets inferred from the layer's own posterior, LatentOutputs.py:20-49): y_tilde_i = d_i a_i.
 // NB regions l0, l0 + stride, ... at once: their loads are issued together (the step is a chain of L2 round trips).
 template <int NB>
@@ -448,20 +454,27 @@ __device__ __forceinline__ void mid2_stats_upper(const ChainModel &m, const Chai
 #pragma unroll
     for (int q = 0; q < NB; ++q) quad[q] = 0.0;
     if (__any_sync(kFull, any)) {      // dA^T G dA (zero in the inert regime of the published model: skipped)
+        // column `lane` of G of each region, all 32 loads of a column in flight at once; those of region q + 1 are issued
+        // before the FMA chain of region q, so the batch costs about one L2 round trip instead of one per region
+        double g[2][32];
 #pragma unroll
-        for (int q = 0; q < NB; ++q) {
-            const double dA0 = ao[q].x - an[q].x, dA1 = ao[q].y - an[q].y;
-            const double *G = ly.gram + (size_t)(live[q] ? l0 + q * stride : 0) * M * M;
-            double g[32];      // column `lane` of G: all its loads in flight at once (one L2 round trip per region)
+        for (int q = 0; q <= NB; ++q) {
+            if (q < NB) {
+                const double *G = ly.gram + (size_t)(live[q] ? l0 + q * stride : 0) * M * M;
 #pragma unroll
-            for (int k = 0; k < 32; ++k) g[k] = (on && live[q] && k < M) ? __ldg(G + (size_t)k * M + lane) : 0.0;
-            double t0 = 0.0, t1 = 0.0;
-#pragma unroll
-            for (int k = 0; k < 32; ++k) {
-                t0 = fma(g[k], __shfl_sync(kFull, dA0, k), t0);
-                t1 = fma(g[k], __shfl_sync(kFull, dA1, k), t1);
+                for (int k = 0; k < 32; ++k) g[q & 1][k] = (on && live[q] && k < M) ? __ldg(G + (size_t)k * M + lane) : 0.0;
             }
-            quad[q] = dA0 * t0 + dA1 * t1;
+            if (q > 0) {
+                const int p = q - 1;
+                const double dA0 = ao[p].x - an[p].x, dA1 = ao[p].y - an[p].y;
+                double t0 = 0.0, t1 = 0.0;
+#pragma unroll
+                for (int k = 0; k < 32; ++k) {
+                    t0 = fma(g[p & 1][k], __shfl_sync(kFull, dA0, k), t0);
+                    t1 = fma(g[p & 1][k], __shfl_sync(kFull, dA1, k), t1);
+                }
+                quad[p] = dA0 * t0 + dA1 * t1;
+            }
         }
         wsum_n<NB>(quad);
     }
@@ -920,20 +933,15 @@ __device__ __forceinline__ void shared_step(const ChainModel &m, ChainSmem &sm, 
     if (tid == 0) PROF(5);
 }
 
-// Worker steps of one warp for a whole layer, NB regions at a time (NB by the regions per worker warp).
+// Worker steps of one warp for a whole layer: regions ww, ww + n_workers, ..., a batch at a time (the order in which
+// a warp adds its regions into acc does not depend on the batch size).
 // (Inlined at their three call sites: as separate functions they cost 4 % - the calls spill around the 255-register solver.)
 __device__ __forceinline__ void layer_mid1(const ChainModel &m, int j, int ww, int n_workers, int lane, const double *ardMean, double (&acc)[7]) {
     const ChainLayer &ly = m.layer[j];
     if (j == 0) {
         for (int l = ww; l < ly.R; l += n_workers) mid1_layer0(m, ly, l, lane, ardMean, acc);
-    } else if (ly.R <= n_workers) {
-        if (ww < ly.R) mid1_upper<1>(m, ly, ww, n_workers, lane, ardMean, acc);
-    } else if (ly.R <= 2 * n_workers) {
-        mid1_upper<2>(m, ly, ww, n_workers, lane, ardMean, acc);
-    } else if (ly.R <= 4 * n_workers) {
-        mid1_upper<4>(m, ly, ww, n_workers, lane, ardMean, acc);
     } else {
-        for (int l = ww; l < ly.R; l += 8 * n_workers) mid1_upper<8>(m, ly, l, n_workers, lane, ardMean, acc);
+        for (int l = ww; l < ly.R; l += kMid1Batch * n_workers) mid1_upper<kMid1Batch>(m, ly, l, n_workers, lane, ardMean, acc);
     }
 }
 
@@ -941,12 +949,8 @@ __device__ __forceinline__ void layer_finish(const ChainModel &m, int j, int ww,
     const ChainLayer &ly = m.layer[j];
     if (j == 0) {
         for (int l = ww; l < ly.R; l += n_workers) mid2_stats_layer0(m, ly, l, lane, cov);
-    } else if (ly.R <= n_workers) {
-        if (ww < ly.R) mid2_stats_upper<1>(m, ly, ww, n_workers, lane, cov);
-    } else if (ly.R <= 2 * n_workers) {
-        mid2_stats_upper<2>(m, ly, ww, n_workers, lane, cov);
     } else {
-        for (int l = ww; l < ly.R; l += 4 * n_workers) mid2_stats_upper<4>(m, ly, l, n_workers, lane, cov);
+        for (int l = ww; l < ly.R; l += kFinishBatch * n_workers) mid2_stats_upper<kFinishBatch>(m, ly, l, n_workers, lane, cov);
     }
 }
 
@@ -1063,7 +1067,9 @@ __global__ void __launch_bounds__(kChainThreads, 1) k_ci_sweep(const ChainModel 
         if (worker && j > 0) {   // S2 and P4 / P5 of layer j - 1 in the background of the chain (C >= 2) / of the solve (C == 1)
             const long long tf = clock64();
             if (early && j > 1) bar_wait(&sm.barF, (unsigned)(j - 2) & 1u);   // F(j - 2): the moments of the coarser layers are complete
+            if (ts && lane == 0) atomicMin(&ts[((j - 1) * 4 + 0) * 2], gtimer());
             layer_finish(m, j - 1, ww, n_workers, lane, sm.loc[(j - 1) & 1]);
+            if (ts && lane == 0) atomicMax(&ts[((j - 1) * 4 + 0) * 2 + 1], gtimer());
             if (early && j < J) {                                             // F(j - 1) to every worker CTA
                 worker_bar(wthreads);
                 if (warp == 0 && lane + 1 < (int)C) bar_arrive_remote(remote_addr(smem_addr(&sm.barF), lane + 1));
@@ -1100,7 +1106,6 @@ __global__ void __launch_bounds__(kChainThreads, 1) k_ci_sweep(const ChainModel 
         if (rank == 0 && warp == 1 && lane < M) sm.skNext[lane] = -sm.logC[lane] + sm.shape[lane] * log(sm.scale[lane]) - lgamma(sm.shape[lane]);
         if (worker) {
             const bool stamp = ww == 0 && lane == 0;
-            if (ts && stamp) atomicMin(&ts[(j * 4 + 1) * 2], gtimer());
             if (stamp) PROF(10);
             double *loc = sm.loc[j & 1];
             if (early) {
@@ -1111,6 +1116,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) k_ci_sweep(const ChainModel 
                 worker_bar(wthreads);
             }
             if (stamp) PROF(11);
+            if (ts && lane == 0) atomicMin(&ts[(j * 4 + 1) * 2], gtimer());
 #pragma unroll
             for (int q = 0; q < 7; ++q) acc[q] = 0.0;
             if (j + 1 < J) {
@@ -1119,7 +1125,7 @@ __global__ void __launch_bounds__(kChainThreads, 1) k_ci_sweep(const ChainModel 
                 publish_sums(sm, acc, early, rank, warp, lane, w0, wt, wthreads);
             }
             if (stamp) PROF(13);
-            if (ts && stamp) atomicMax(&ts[(j * 4 + 1) * 2 + 1], gtimer());
+            if (ts && lane == 0) atomicMax(&ts[(j * 4 + 1) * 2 + 1], gtimer());
             if (stamp) PROF(14);
         }
     }
@@ -1150,6 +1156,17 @@ __global__ void __launch_bounds__(kChainThreads, 1) k_ci_sweep(const ChainModel 
             if ((t & 31) < M) m.omegaEta[(t >> 5) * 64 + (t & 31)] = log(sm.vout[t >> 5][t & 31]) - sm.cshift[t >> 5][t & 31];
         if (tid == 0) atomicAdd(m.chol_count, (unsigned long long)sm.nchol);
         if (ts && tid == 0) atomicMax(&ts[((J - 1) * 4 + 1) * 2 + 1], gtimer());
+    }
+    // timeline, slots kind 2 of layers 0 and 1: the exits of the warps of CTA 0 and of every warp of the cluster (the
+    // workers' finish of the last layers runs after the chain)
+    if (ts && lane == 0) {
+        const unsigned long long t = gtimer();
+        if (rank == 0) {
+            atomicMin(&ts[(0 * 4 + 2) * 2], t);
+            atomicMax(&ts[(0 * 4 + 2) * 2 + 1], t);
+        }
+        atomicMin(&ts[(1 * 4 + 2) * 2], t);
+        atomicMax(&ts[(1 * 4 + 2) * 2 + 1], t);
     }
 }
 
