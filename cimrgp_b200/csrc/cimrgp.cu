@@ -119,11 +119,9 @@ struct mrgp_handle {
     bool elbo_no_sync = false;
     bool prefetch_pending = false, y_free_recorded = false;
     cudaStream_t side2 = nullptr;    // layer 0's phase B beside the chain of layer 1 (closed-form ci sweeps)
-    bool b0_pending = false;
     cudaGraph_t graph = nullptr;
     cudaGraphExec_t graph_exec = nullptr;
     int64_t launches = 0, launches_per_sweep = 0, sweeps_done = 0;
-    bool capturing = false;
     bool timeline = false;
     double *x_all = nullptr;         // sharded handles: inputs of ALL ranks (mrgp_set_all_inputs_host), else unused
     bool have_x_all = false;
@@ -138,7 +136,6 @@ struct mrgp_handle {
     double *chain_guard = nullptr, *chain_prof = nullptr, *chain_tables = nullptr;
     double chain_guard_threshold = kChainGuard;   // MRGP_CHAIN_GUARD overrides (tests of the streamed fallback)
     bool chain_prof_on = false;      // MRGP_CHAIN_PROF=1: SM-clock stamps of the fused sweep (field 54)
-    const unsigned int *gate_next = nullptr;   // gate of the next phase-B launch (streamed fallback of the fused sweep)
     bool elbo_args_valid = false;    // the per-layer argument blocks of k_elbo on the device match generation / sweeps_done
     uint64_t elbo_args_key = 0;
     bool chain_uploaded = false;     // the device descriptor matches the current pointers (reset by drop_graph)
@@ -472,7 +469,6 @@ StreamArgs stream_args(mrgp_handle *h, int j) {
     a.region_run = d.region_run;
     a.offsets = d.offsets;
     a.R = h->plan[j].R;
-    a.gate = h->gate_next;
     a.n_basis = h->cfg.n_basis;
     a.infer = (h->cfg.mode == MRGP_MODE_CI && j > 0) ? 1 : 0;
     a.fuse_tail = 0;
@@ -628,7 +624,7 @@ cudaError_t set_smem(K kernel, size_t bytes) {
 }
 
 template <int M>
-cudaError_t launch_phase_a(mrgp_handle *h, const StreamArgs &a, bool infer, bool latent) {
+cudaError_t launch_phase_a(mrgp_handle *h, cudaStream_t stream, const StreamArgs &a, bool infer, bool latent) {
     constexpr int DY = 2;
     dim3 grid(h->n_ctas), block(kThreads);
 #define LA(I, L)                                                                                               \
@@ -636,7 +632,7 @@ cudaError_t launch_phase_a(mrgp_handle *h, const StreamArgs &a, bool infer, bool
         const size_t smem = (size_t)(kStages * TileLayout<DY, !(I), (L), false>::kDoubles + kRedSmemDoubles) * sizeof(double); \
         cudaError_t e = set_smem(k_phase_a<DY, M, I, L>, smem);                                                \
         if (e != cudaSuccess) return e;                                                                        \
-        k_phase_a<DY, M, I, L><<<grid, block, smem, h->stream>>>(a);                                           \
+        k_phase_a<DY, M, I, L><<<grid, block, smem, stream>>>(a);                                              \
     }
     if (infer)
         LA(true, true)
@@ -649,7 +645,7 @@ cudaError_t launch_phase_a(mrgp_handle *h, const StreamArgs &a, bool infer, bool
 }
 
 template <int M>
-cudaError_t launch_phase_b(mrgp_handle *h, const StreamArgs &a, bool infer, bool latent, bool prop) {
+cudaError_t launch_phase_b(mrgp_handle *h, cudaStream_t stream, const StreamArgs &a, bool infer, bool latent, bool prop) {
     constexpr int DY = 2;
     dim3 grid(h->n_ctas), block(kThreadsB);
 #define LB(I, L, P)                                                                                         \
@@ -657,7 +653,7 @@ cudaError_t launch_phase_b(mrgp_handle *h, const StreamArgs &a, bool infer, bool
         const size_t smem = (size_t)(kStages * TileLayout<DY, !(I), (L), (L)>::kDoubles) * sizeof(double);  \
         cudaError_t e = set_smem(k_phase_b<DY, M, I, L, P>, smem);                                          \
         if (e != cudaSuccess) return e;                                                                     \
-        k_phase_b<DY, M, I, L, P><<<grid, block, smem, h->stream>>>(a);                                     \
+        k_phase_b<DY, M, I, L, P><<<grid, block, smem, stream>>>(a);                                        \
     }
     if (infer) {
         if (prop)
@@ -680,10 +676,10 @@ cudaError_t launch_phase_b(mrgp_handle *h, const StreamArgs &a, bool infer, bool
 }
 
 template <int M>
-cudaError_t launch_phi2sum(mrgp_handle *h, const StreamArgs &a) {
+cudaError_t launch_phi2sum(mrgp_handle *h, cudaStream_t stream, const StreamArgs &a) {
     cudaError_t e = set_smem(k_phi2sum<M>, kRedSmemBytes);
     if (e != cudaSuccess) return e;
-    k_phi2sum<M><<<h->n_ctas, kThreads, kRedSmemBytes, h->stream>>>(a);
+    k_phi2sum<M><<<h->n_ctas, kThreads, kRedSmemBytes, stream>>>(a);
     return cudaGetLastError();
 }
 
@@ -710,22 +706,23 @@ int check_ready(mrgp_handle *h, int layer, bool need_state) {
     return MRGP_OK;
 }
 
-void count(mrgp_handle *h, int n = 1) {
-    if (h->capturing)
-        h->launches_per_sweep += n;
-    else
-        h->launches += n;
-}
+// Where a helper enqueues its work and which counter its kernel launches add to: the handle's stream and
+// mrgp_handle::launches outside a sweep; a captured sweep counts into its own per-sweep count, and a branch of a sweep
+// onto another stream keeps the counter of the sweep.
+struct Launch {
+    cudaStream_t stream;
+    int64_t *count;
+};
 
 // ---- the phases ---------------------------------------------------------------------------------
-int do_phase_a(mrgp_handle *h, int j) {
+int do_phase_a(mrgp_handle *h, const Launch &L, int j) {
     const bool fi = h->cfg.mode == MRGP_MODE_FI;
     const bool infer = !fi && j > 0, latent = j > 0;
     StreamArgs a = stream_args(h, j);
     cudaError_t e = cudaErrorInvalidValue;
-    DISPATCH_M(h->cfg.n_basis, e = launch_phase_a<MM>(h, a, infer, latent));
+    DISPATCH_M(h->cfg.n_basis, e = launch_phase_a<MM>(h, L.stream, a, infer, latent));
     CK(e);
-    count(h);
+    *L.count += 1;
     return MRGP_OK;
 }
 
@@ -741,12 +738,12 @@ int max_region_runs(const LayerPlan &lp) {
     return m;
 }
 
-int do_mid_ci(mrgp_handle *h, int j, bool fork_omega, bool zero_T = false);
+int do_mid_ci(mrgp_handle *h, const Launch &L, int j, bool fork_omega, bool zero_T = false);
 
-int do_axis_update(mrgp_handle *h, int j, bool fork_omega, bool zero_T = false) {
+int do_axis_update(mrgp_handle *h, const Launch &L, int j, bool fork_omega, bool zero_T = false) {
     const bool fi = h->cfg.mode == MRGP_MODE_FI;
     const int M = h->cfg.n_basis, DY = h->cfg.dy;
-    if (!fi) return do_mid_ci(h, j, fork_omega, zero_T);
+    if (!fi) return do_mid_ci(h, L, j, fork_omega, zero_T);
     RegionArgs a = region_args(h, j);
     const LayerPlan &lp = h->plan[j];
     {
@@ -755,19 +752,19 @@ int do_axis_update(mrgp_handle *h, int j, bool fork_omega, bool zero_T = false) 
         const int slices = threads / nval;
         const size_t smem = (size_t)(slices * nval + nv) * sizeof(double);
         CK(set_smem(k_reduce_scale<2>, smem));
-        k_reduce_scale<2><<<lp.R, threads, smem, h->stream>>>(a);
+        k_reduce_scale<2><<<lp.R, threads, smem, L.stream>>>(a);
         CK(cudaGetLastError());
-        count(h);
+        *L.count += 1;
     }
     return MRGP_OK;
 }
 
-int do_mid_ci(mrgp_handle *h, int j, bool fork_omega, bool zero_T) {
+int do_mid_ci(mrgp_handle *h, const Launch &L, int j, bool fork_omega, bool zero_T) {
     const int M = h->cfg.n_basis;
     RegionArgs a = region_args(h, j);
     a.zero_T = zero_T ? 1 : 0;
     const LayerPlan &lp = h->plan[j];
-    if (fork_omega && j > 0) CK(cudaStreamWaitEvent(h->stream, h->ev_ard[j - 1], 0));   // k_mid1 reads ard_mean
+    if (fork_omega && j > 0) CK(cudaStreamWaitEvent(L.stream, h->ev_ard[j - 1], 0));   // k_mid1 reads ard_mean
     int n_partials = 1;
     {
         const int mr = h->sharded ? 1 : max_region_runs(lp);
@@ -780,15 +777,15 @@ int do_mid_ci(mrgp_handle *h, int j, bool fork_omega, bool zero_T) {
         const int nvp = (M * 3 + 31) & ~31, nvwp = (M * 4 + 31) & ~31;
         const size_t smem1 = (size_t)(2 * 32 * M * 4 + nvp + nvwp) * sizeof(double);
         CK(set_smem(k_mid1<2>, smem1));
-        k_mid1<2><<<nb, kMidThreads, smem1, h->stream>>>(a, lpi, rpc);
+        k_mid1<2><<<nb, kMidThreads, smem1, L.stream>>>(a, lpi, rpc);
         CK(cudaGetLastError());
-        count(h);
+        *L.count += 1;
         n_partials = nb;
         // The critical chain of the sweep is omega(j-1) -> axis / ARD update and table (k_ard) -> omega(j): k_ard only
         // needs the region sums of k_mid1, so it is forked here and runs beside k_mid2 (S2 of the regions).
-        cudaStream_t st = h->stream;
+        cudaStream_t st = L.stream;
         if (fork_omega) {
-            CK(cudaEventRecord(h->ev_fork[j], h->stream));
+            CK(cudaEventRecord(h->ev_fork[j], L.stream));
             CK(cudaStreamWaitEvent(h->side, h->ev_fork[j], 0));
             st = h->side;
         }
@@ -803,14 +800,14 @@ int do_mid_ci(mrgp_handle *h, int j, bool fork_omega, bool zero_T) {
         const int rpc2 = (lp.R + nb2 - 1) / nb2;
         nb2 = (lp.R + rpc2 - 1) / rpc2;
         const size_t smem2 = (size_t)(std::max(33 * M, M * M + 4 * M + 3 * nvp) + 4 * M) * sizeof(double);
-        if (fork_omega && j > 0) CK(cudaStreamWaitEvent(h->stream, h->ev_join[j - 1], 0));   // k_mid2 reads omega
+        if (fork_omega && j > 0) CK(cudaStreamWaitEvent(L.stream, h->ev_join[j - 1], 0));   // k_mid2 reads omega
         CK(set_smem(k_mid2<2>, smem2));
-        k_mid2<2><<<nb2, kMidThreads, smem2, h->stream>>>(a, rpc2, nb);
+        k_mid2<2><<<nb2, kMidThreads, smem2, L.stream>>>(a, rpc2, nb);
         CK(cudaGetLastError());
-        count(h);
+        *L.count += 1;
         if (fork_omega) {
             // k_scale_warp overwrites omega, which k_mid2 reads
-            CK(cudaEventRecord(h->ev_mid2[j], h->stream));
+            CK(cudaEventRecord(h->ev_mid2[j], L.stream));
             CK(cudaStreamWaitEvent(h->side, h->ev_mid2[j], 0));
         } else {
             CK(set_smem(k_ard, smem));
@@ -831,51 +828,53 @@ int do_mid_ci(mrgp_handle *h, int j, bool fork_omega, bool zero_T) {
             k_scale<<<1, kOmegaThreads, smem, st>>>(a);
         }
         CK(cudaGetLastError());
-        count(h, 2);
+        *L.count += 2;
         if (fork_omega) CK(cudaEventRecord(h->ev_join[j], h->side));
     }
     return MRGP_OK;
 }
 
-int do_bias_noise_shared(mrgp_handle *h, int j);
+int do_bias_noise_shared(mrgp_handle *h, const Launch &L, int j);
 
-int do_phase_b(mrgp_handle *h, int j, bool fuse_tail, int prop_override = -1) {
+// `gate`: when not null the kernel runs only if *gate != 0 (the streamed fallback of the fused sweep).
+int do_phase_b(mrgp_handle *h, const Launch &L, int j, bool fuse_tail, int prop_override = -1, const unsigned int *gate = nullptr) {
     const bool fi = h->cfg.mode == MRGP_MODE_FI;
     const bool infer = !fi && j > 0, latent = j > 0;
     const bool prop = prop_override < 0 ? (j + 1 < h->cfg.n_layers) : (prop_override != 0);
     StreamArgs a = stream_args(h, j);
     a.fuse_tail = fuse_tail ? 1 : 0;
+    a.gate = gate;
     cudaError_t e = cudaErrorInvalidValue;
-    DISPATCH_M(h->cfg.n_basis, e = launch_phase_b<MM>(h, a, infer, latent, prop));
+    DISPATCH_M(h->cfg.n_basis, e = launch_phase_b<MM>(h, L.stream, a, infer, latent, prop));
     CK(e);
-    count(h);
-    return fuse_tail ? do_bias_noise_shared(h, j) : MRGP_OK;
+    *L.count += 1;
+    return fuse_tail ? do_bias_noise_shared(h, L, j) : MRGP_OK;
 }
 
 // Second stage of the bias / noise update when noise or bias is shared by the regions of a layer.
-int do_bias_noise_shared(mrgp_handle *h, int j) {
+int do_bias_noise_shared(mrgp_handle *h, const Launch &L, int j) {
     if (h->cfg.noise_region_specific && h->cfg.bias_region_specific) return MRGP_OK;
     StreamArgs a = stream_args(h, j);
-    k_bias_noise_shared<2><<<1, 256, 0, h->stream>>>(a);
+    k_bias_noise_shared<2><<<1, 256, 0, L.stream>>>(a);
     CK(cudaGetLastError());
-    count(h);
+    *L.count += 1;
     return MRGP_OK;
 }
 
-int do_bias_noise(mrgp_handle *h, int j) {
+int do_bias_noise(mrgp_handle *h, const Launch &L, int j) {
     StreamArgs a = stream_args(h, j);
     if (h->sharded) {
         a.region_run = h->dev[j].ident_run;
         a.part = h->xchg;
     }
-    k_bias_noise<2><<<std::max(1, std::min(32, (h->plan[j].R + 7) / 8)), kThreadsB, 0, h->stream>>>(a);
+    k_bias_noise<2><<<std::max(1, std::min(32, (h->plan[j].R + 7) / 8)), kThreadsB, 0, L.stream>>>(a);
     CK(cudaGetLastError());
-    count(h);
-    return do_bias_noise_shared(h, j);
+    *L.count += 1;
+    return do_bias_noise_shared(h, L, j);
 }
 
 // One exchange over peer memory: local dense sums -> arena slot, publish, reduce over the owning ranks -> h->xchg.
-int do_exchange(mrgp_handle *h, int j, int slot, int nv, bool is_max) {
+int do_exchange(mrgp_handle *h, const Launch &L, int j, int slot, int nv, bool is_max) {
     if (!h->comm.ready) return fail(h, MRGP_ESTATE, "no peer exchange bound: mrgp_comm_export / mrgp_comm_bind first");
     const LayerPlan &lp = h->plan[j];
     LayerDev &d = h->dev[j];
@@ -883,47 +882,47 @@ int do_exchange(mrgp_handle *h, int j, int slot, int nv, bool is_max) {
     (void)slot;   // the arena slot follows the exchange number on the device (k_comm_sums_signal)
     if (h->part_stride > 256) return fail(h, MRGP_EINVAL, "exchange rows of more than 256 values are not supported");
     if (is_max)
-        k_comm_sums_signal<true><<<lp.R, 256, 0, h->stream>>>(h->comm.args, d.region_run, h->part, h->part_stride, nv, h->comm.arena, h->comm.counter);
+        k_comm_sums_signal<true><<<lp.R, 256, 0, L.stream>>>(h->comm.args, d.region_run, h->part, h->part_stride, nv, h->comm.arena, h->comm.counter);
     else
-        k_comm_sums_signal<false><<<lp.R, 256, 0, h->stream>>>(h->comm.args, d.region_run, h->part, h->part_stride, nv, h->comm.arena, h->comm.counter);
+        k_comm_sums_signal<false><<<lp.R, 256, 0, L.stream>>>(h->comm.args, d.region_run, h->part, h->part_stride, nv, h->comm.arena, h->comm.counter);
     CK(cudaGetLastError());
     const int grid = std::max(1, std::min(96, (total + 255) / 256));
     if (is_max)
-        k_comm_reduce<true><<<grid, 256, 0, h->stream>>>(h->comm.args, d.offsets, lp.R, h->part_stride, nv, h->xchg);
+        k_comm_reduce<true><<<grid, 256, 0, L.stream>>>(h->comm.args, d.offsets, lp.R, h->part_stride, nv, h->xchg);
     else
-        k_comm_reduce<false><<<grid, 256, 0, h->stream>>>(h->comm.args, d.offsets, lp.R, h->part_stride, nv, h->xchg);
+        k_comm_reduce<false><<<grid, 256, 0, L.stream>>>(h->comm.args, d.offsets, lp.R, h->part_stride, nv, h->xchg);
     CK(cudaGetLastError());
-    count(h, 2);
+    *L.count += 2;
     return MRGP_OK;
 }
 
 template <int M>
-cudaError_t launch_objective(mrgp_handle *h, const IntervalArgs &q, bool infer, bool latent) {
+cudaError_t launch_objective(mrgp_handle *h, cudaStream_t stream, const IntervalArgs &q, bool infer, bool latent) {
     dim3 grid(h->n_ctas), block(kThreads);
     if (infer)
-        k_interval_objective<2, M, true, true><<<grid, block, 0, h->stream>>>(q);
+        k_interval_objective<2, M, true, true><<<grid, block, 0, stream>>>(q);
     else if (latent)
-        k_interval_objective<2, M, false, true><<<grid, block, 0, h->stream>>>(q);
+        k_interval_objective<2, M, false, true><<<grid, block, 0, stream>>>(q);
     else
-        k_interval_objective<2, M, false, false><<<grid, block, 0, h->stream>>>(q);
+        k_interval_objective<2, M, false, false><<<grid, block, 0, stream>>>(q);
     return cudaGetLastError();
 }
 
 template <int M>
-cudaError_t launch_elbo_sums(mrgp_handle *h, const IntervalArgs &q, bool infer, bool latent) {
+cudaError_t launch_elbo_sums(mrgp_handle *h, cudaStream_t stream, const IntervalArgs &q, bool infer, bool latent) {
     dim3 grid(h->n_ctas), block(kThreads);
     if (infer)
-        k_adaptive_elbo_sums<2, M, true, true><<<grid, block, 0, h->stream>>>(q);
+        k_adaptive_elbo_sums<2, M, true, true><<<grid, block, 0, stream>>>(q);
     else if (latent)
-        k_adaptive_elbo_sums<2, M, false, true><<<grid, block, 0, h->stream>>>(q);
+        k_adaptive_elbo_sums<2, M, false, true><<<grid, block, 0, stream>>>(q);
     else
-        k_adaptive_elbo_sums<2, M, false, false><<<grid, block, 0, h->stream>>>(q);
+        k_adaptive_elbo_sums<2, M, false, false><<<grid, block, 0, stream>>>(q);
     return cudaGetLastError();
 }
 
 // B1: BasisInterval.learn for one layer (BasisInterval.py:18-134), then the rebuild of lambda, S and sum phi^2
 // (MRGP.py:640-641).  ci mode only (MRGP.py:108-109 switches it off for fi).
-int do_learn_intervals(mrgp_handle *h, int j) {
+int do_learn_intervals(mrgp_handle *h, const Launch &L, int j) {
     LayerDev &d = h->dev[j];
     const LayerPlan &lp = h->plan[j];
     const int M = h->cfg.n_basis;
@@ -948,9 +947,9 @@ int do_learn_intervals(mrgp_handle *h, int j) {
     b.xatol = 1e-5;
     b.maxfun = 500;
     const int total = lp.R * M;
-    k_brent_start<<<(total + 127) / 128, 128, 0, h->stream>>>(b, d.absx, d.ad_lo, d.ad_hi, d.A, d.cm2, d.wq);
+    k_brent_start<<<(total + 127) / 128, 128, 0, L.stream>>>(b, d.absx, d.ad_lo, d.ad_hi, d.A, d.cm2, d.wq);
     CK(cudaGetLastError());
-    count(h);
+    *L.count += 1;
     IntervalArgs q{};
     q.s = stream_args(h, j);
     q.trial_inv2L = d.trial_inv2L;
@@ -959,29 +958,29 @@ int do_learn_intervals(mrgp_handle *h, int j) {
     q.bias_old = d.bias_prev;
     for (int it = 0; it < h->ad_iters; ++it) {
         cudaError_t e = cudaErrorInvalidValue;
-        DISPATCH_M(M, e = launch_objective<MM>(h, q, infer, latent));
+        DISPATCH_M(M, e = launch_objective<MM>(h, L.stream, q, infer, latent));
         CK(e);
         b.first = (it == 0) ? 1 : 0;
-        k_brent_step<<<(lp.R + 3) / 4, 128, 0, h->stream>>>(b);
+        k_brent_step<<<(lp.R + 3) / 4, 128, 0, L.stream>>>(b);
         CK(cudaGetLastError());
-        count(h, 2);
+        *L.count += 2;
     }
-    k_brent_finish<<<(lp.R + 127) / 128, 128, 0, h->stream>>>(b, d.L, h->brent_fail);
+    k_brent_finish<<<(lp.R + 127) / 128, 128, 0, L.stream>>>(b, d.L, h->brent_fail);
     CK(cudaGetLastError());
     // the targets of this step were inferred with the current basis: keep it for the lower bound
-    CK(cudaMemcpyAsync(d.inv2L_old, d.inv2L, lp.R * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
-    CK(cudaMemcpyAsync(d.rsqrtL_old, d.rsqrtL, lp.R * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+    CK(cudaMemcpyAsync(d.inv2L_old, d.inv2L, lp.R * sizeof(double), cudaMemcpyDeviceToDevice, L.stream));
+    CK(cudaMemcpyAsync(d.rsqrtL_old, d.rsqrtL, lp.R * sizeof(double), cudaMemcpyDeviceToDevice, L.stream));
     RegionArgs ra = region_args(h, j);
     ra.L_given = 1;
-    k_region_setup<<<(lp.R + 7) / 8, 256, 0, h->stream>>>(ra);
+    k_region_setup<<<(lp.R + 7) / 8, 256, 0, L.stream>>>(ra);
     CK(cudaGetLastError());
     StreamArgs sa = stream_args(h, j);
     cudaError_t e = cudaErrorInvalidValue;
-    DISPATCH_M(M, e = launch_phi2sum<MM>(h, sa));
+    DISPATCH_M(M, e = launch_phi2sum<MM>(h, L.stream, sa));
     CK(e);
-    k_reduce_d<<<lp.R, 64, 0, h->stream>>>(ra);
+    k_reduce_d<<<lp.R, 64, 0, L.stream>>>(ra);
     CK(cudaGetLastError());
-    count(h, 4);
+    *L.count += 4;
     // data-term sums of the lower bound with the re-learnt basis (before the propagation overwrites g, h)
     {
         IntervalArgs qe{};
@@ -991,14 +990,14 @@ int do_learn_intervals(mrgp_handle *h, int j) {
         qe.w = nullptr;
         qe.bias_old = d.bias_prev;
         cudaError_t ee = cudaErrorInvalidValue;
-        DISPATCH_M(M, ee = launch_elbo_sums<MM>(h, qe, infer, latent));
+        DISPATCH_M(M, ee = launch_elbo_sums<MM>(h, L.stream, qe, infer, latent));
         CK(ee);
         StreamArgs se = stream_args(h, j);
         se.sums_only = 1;
         se.sumsB = d.sumsE;
-        k_bias_noise<2><<<std::max(1, std::min(32, (lp.R + 7) / 8)), kThreadsB, 0, h->stream>>>(se);
+        k_bias_noise<2><<<std::max(1, std::min(32, (lp.R + 7) / 8)), kThreadsB, 0, L.stream>>>(se);
         CK(cudaGetLastError());
-        count(h, 2);
+        *L.count += 2;
     }
     return MRGP_OK;
 }
@@ -1029,47 +1028,47 @@ bool use_fused(const mrgp_handle *h) {
 }
 
 template <int M>
-int launch_build_invariants(mrgp_handle *h, int j) {
+int launch_build_invariants(mrgp_handle *h, const Launch &L, int j) {
     LayerDev &d = h->dev[j];
     const LayerPlan &lp = h->plan[j];
     const int splits = build_splits(lp.R), blocks = lp.R * splits;
     constexpr int NP = M * (M + 1) / 2;
     CK(cudaFuncSetAttribute(k_build_gram<M>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
     const double *xg = h->sharded ? h->x_all : h->x;   // indexed by the global sample number
-    k_build_gram<M><<<blocks, 256, 0, h->stream>>>(xg, d.offsets, d.inv2L, d.rsqrtL, splits, h->build_part);
+    k_build_gram<M><<<blocks, 256, 0, L.stream>>>(xg, d.offsets, d.inv2L, d.rsqrtL, splits, h->build_part);
     CK(cudaGetLastError());
-    k_reduce_gram<<<(lp.R * (NP + M) + 255) / 256, 256, 0, h->stream>>>(h->build_part, splits, lp.R, h->cfg.n_basis, M, d.gram, d.sumPhi);
+    k_reduce_gram<<<(lp.R * (NP + M) + 255) / 256, 256, 0, L.stream>>>(h->build_part, splits, lp.R, h->cfg.n_basis, M, d.gram, d.sumPhi);
     CK(cudaGetLastError());
-    count(h, 2);
+    *L.count += 2;
     if (j > 0) {
         EvalArgs ea{};
         int rc = fill_eval_layers(h, ea, j, nullptr);
         if (rc) return rc;
         const int P = (int)lp.pc_jp.size(), psplits = build_splits(P);
         const PieceTable pt{d.pc_ptr, d.pc_jp, d.pc_anc, d.pc_lo, d.pc_hi, P};
-        k_build_ancD<M><<<P * psplits, 256, 0, h->stream>>>(ea, xg, pt, psplits, h->build_part);
+        k_build_ancD<M><<<P * psplits, 256, 0, L.stream>>>(ea, xg, pt, psplits, h->build_part);
         CK(cudaGetLastError());
-        k_reduce_ancD<<<(P * h->cfg.n_basis + 255) / 256, 256, 0, h->stream>>>(h->build_part, psplits, P, h->cfg.n_basis, M, d.ancD);
+        k_reduce_ancD<<<(P * h->cfg.n_basis + 255) / 256, 256, 0, L.stream>>>(h->build_part, psplits, P, h->cfg.n_basis, M, d.ancD);
         CK(cudaGetLastError());
-        count(h, 2);
+        *L.count += 2;
     }
     d.inv_built = true;
     return MRGP_OK;
 }
 
-int build_invariants(mrgp_handle *h) {
+int build_invariants(mrgp_handle *h, const Launch &L) {
     const bool fused = use_fused(h);
     if (!use_closed_form(h) && !fused) return MRGP_OK;
     for (int j = fused ? 0 : 1; j < h->cfg.n_layers; ++j) {
         if (h->dev[j].inv_built) continue;
         int rc = MRGP_EINVAL;
-        DISPATCH_M(h->cfg.n_basis, rc = launch_build_invariants<MM>(h, j));
+        DISPATCH_M(h->cfg.n_basis, rc = launch_build_invariants<MM>(h, L, j));
         if (rc) return rc;
     }
     return MRGP_OK;
 }
 
-int do_stats_b(mrgp_handle *h, int j) {
+int do_stats_b(mrgp_handle *h, const Launch &L, int j) {
     LayerDev &d = h->dev[j];
     StatsBArgs q{};
     q.p = stream_args(h, j);
@@ -1085,23 +1084,21 @@ int do_stats_b(mrgp_handle *h, int j) {
     q.d = d.d;
     q.cm2 = d.cm2;
     CK(cudaFuncSetAttribute(k_stats_b<2>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    k_stats_b<2><<<(h->plan[j].R + 7) / 8, 256, 0, h->stream>>>(q);
+    k_stats_b<2><<<(h->plan[j].R + 7) / 8, 256, 0, L.stream>>>(q);
     CK(cudaGetLastError());
-    count(h);
-    return do_bias_noise_shared(h, j);
+    *L.count += 1;
+    return do_bias_noise_shared(h, L, j);
 }
-
-int do_exchange(mrgp_handle *h, int j, int slot, int nv, bool is_max);
 
 // Sufficient statistics of the observations for layer 0 of the fused sweep: Phi^T y, sum y, sum |y|^2 per region
 // (one pass over x and y; again whenever y, x or the intervals of layer 0 change).
 template <int M>
-cudaError_t launch_ystats(mrgp_handle *h, const StreamArgs &a) {
+cudaError_t launch_ystats(mrgp_handle *h, cudaStream_t stream, const StreamArgs &a) {
     constexpr int DY = 2;
     const size_t smem = (size_t)(kStages * TileLayout<DY, true, false, false>::kDoubles + kRedSmemDoubles) * sizeof(double);
     cudaError_t e = set_smem(k_ystats<DY, M>, smem);
     if (e != cudaSuccess) return e;
-    k_ystats<DY, M><<<h->n_ctas, kThreads, smem, h->stream>>>(a);
+    k_ystats<DY, M><<<h->n_ctas, kThreads, smem, stream>>>(a);
     return cudaGetLastError();
 }
 
@@ -1115,16 +1112,16 @@ bool ystats_small(const mrgp_handle *h) {
     return true;
 }
 
-int do_ystats(mrgp_handle *h) {
+int do_ystats(mrgp_handle *h, const Launch &L) {
     LayerDev &d = h->dev[0];
     const LayerPlan &lp = h->plan[0];
     const int M = h->cfg.n_basis, DY = h->cfg.dy;
     if (ystats_small(h)) {   // one CTA per region of layer 0, straight from the descriptor (the form a batch of series uses)
         int rc = h->chain_uploaded ? MRGP_OK : upload_chain_model(h);
         if (rc) return rc;
-        const int e = launch_ystats_small(chain_solver_size(M), h->chain_ptr_dev, 1, lp.R, h->stream);
+        const int e = launch_ystats_small(chain_solver_size(M), h->chain_ptr_dev, 1, lp.R, L.stream);
         if (e != 0) return fail(h, MRGP_ECUDA, "y statistics launch: %s", cudaGetErrorString((cudaError_t)e));
-        count(h);
+        *L.count += 1;
         h->ystats_valid = true;
         return MRGP_OK;
     }
@@ -1136,21 +1133,21 @@ int do_ystats(mrgp_handle *h) {
     a.yc_out = d.yc;
     a.ysum_out = d.ysum;
     cudaError_t e = cudaErrorInvalidValue;
-    DISPATCH_M(M, e = launch_ystats<MM>(h, a));
+    DISPATCH_M(M, e = launch_ystats<MM>(h, L.stream, a));
     CK(e);
-    count(h);
+    *L.count += 1;
     if (!fuse) {
         const int32_t *rr = d.region_run;
         const double *part = h->part;
         if (h->sharded) {   // sum the statistics of the ranks' chunks
-            int rc = do_exchange(h, 0, 0, padded_basis(M) * DY + DY + 1, false);
+            int rc = do_exchange(h, L, 0, 0, padded_basis(M) * DY + DY + 1, false);
             if (rc) return rc;
             rr = d.ident_run;
             part = h->xchg;
         }
-        k_reduce_ystats<<<lp.R, 1024, 0, h->stream>>>(rr, part, h->part_stride, lp.R, M, padded_basis(M), DY, d.yc, d.ysum);
+        k_reduce_ystats<<<lp.R, 1024, 0, L.stream>>>(rr, part, h->part_stride, lp.R, M, padded_basis(M), DY, d.yc, d.ysum);
         CK(cudaGetLastError());
-        count(h);
+        *L.count += 1;
     }
     h->ystats_valid = true;
     return MRGP_OK;
@@ -1215,45 +1212,43 @@ int upload_chain_model(mrgp_handle *h) {
     return MRGP_OK;
 }
 
-int do_phase_b(mrgp_handle *h, int j, bool fuse_tail, int prop_override);
-
-int do_fused_sweep(mrgp_handle *h) {
-    const int rc = launch_ci_sweep(chain_solver_size(h->cfg.n_basis), h->chain_ptr_dev, 1, chain_cluster_size(h), h->stream);
+int do_fused_sweep(mrgp_handle *h, const Launch &L) {
+    const int rc = launch_ci_sweep(chain_solver_size(h->cfg.n_basis), h->chain_ptr_dev, 1, chain_cluster_size(h), L.stream);
     if (rc != 0) return fail(h, MRGP_ECUDA, "fused sweep launch: %s", cudaGetErrorString((cudaError_t)rc));
-    count(h);
+    *L.count += 1;
     // Guarded fallback for layer 0: its sum |r|^2 is formed from the sufficient statistics of y as a difference of large
     // terms; when the residual is tiny against sum |y|^2 (ratio below kChainGuard: high-SNR data) the sweep sets the
     // model's status word and the kernel below - a no-op otherwise - takes the statistics of layer 0 by a pass over the
     // samples and repeats its bias / noise update (nothing else of the sweep depends on them).
     if (h->sharded) return MRGP_OK;   // (the sharded handle reports the status; its fallback would need an exchange)
     if (ystats_small(h)) {
-        const int e = launch_l0_fix_small(chain_solver_size(h->cfg.n_basis), h->chain_ptr_dev, 1, h->plan[0].R, h->stream);
+        const int e = launch_l0_fix_small(chain_solver_size(h->cfg.n_basis), h->chain_ptr_dev, 1, h->plan[0].R, L.stream);
         if (e != 0) return fail(h, MRGP_ECUDA, "layer-0 fallback launch: %s", cudaGetErrorString((cudaError_t)e));
-        count(h);
+        *L.count += 1;
         return MRGP_OK;
     }
-    h->gate_next = h->chain_status;
-    const int r2 = do_phase_b(h, 0, true, 0);
-    h->gate_next = nullptr;
-    return r2;
+    return do_phase_b(h, L, 0, true, 0, h->chain_status);
 }
 
-int sweep_once(mrgp_handle *h, bool fork_omega) {
+int sweep_once(mrgp_handle *h, const Launch &L) {
     const int J = h->cfg.n_layers;
     const bool ci = h->cfg.mode == MRGP_MODE_CI;
     const bool closed = use_closed_form(h);
     int rc;
-    if (fork_omega && use_fused(h)) return do_fused_sweep(h);   // the whole sweep is one kernel (csrc/chain.cu)
-    if (fork_omega && ci && h->state_end > h->state_begin) {
+    if (use_fused(h)) return do_fused_sweep(h, L);   // the whole sweep is one kernel (csrc/chain.cu)
+    if (ci && h->state_end > h->state_begin) {
         // the small-matrix state (a few MB) is pulled into L2 by the side stream while layer 0 streams the samples:
         // the short kernels that follow are chains of dependent loads and would otherwise each pay HBM latency
-        CK(cudaEventRecord(h->ev_prefetch, h->stream));
+        CK(cudaEventRecord(h->ev_prefetch, L.stream));
         CK(cudaStreamWaitEvent(h->side, h->ev_prefetch, 0));
         const size_t lines = (h->state_end - h->state_begin + 127) / 128;
         k_prefetch_l2<<<(unsigned)std::min<size_t>((lines + 255) / 256, 1024), 256, 0, h->side>>>(h->ws + h->state_begin, lines);
         CK(cudaGetLastError());
-        count(h);
+        *L.count += 1;
     }
+    // the third stream: layer 0's phase B (b0_forked once it is there), then the closed-form statistics of the layers above
+    const Launch b0{h->side2, L.count};
+    bool b0_forked = false;
     for (int j = 0; j < J; ++j) {
         // ci layers above the first regress on targets inferred from their own posterior, y = Phi A + b + fbar
         // (LatentOutputs.py:20-49), so the residual of the P1 statistics, y - fbar - b - Phi A with the same A and b
@@ -1261,66 +1256,53 @@ int sweep_once(mrgp_handle *h, bool fork_omega) {
         // would add up those zeros (plus roundoff) is not launched; mrgp_phase_a still runs it on request and
         // MRGP_STREAM_ALL=1 puts it back into the sweep.
         const bool zero_T = ci && j > 0 && h->inferred_shortcut;
-        if (!zero_T && (rc = do_phase_a(h, j))) return rc;
+        if (!zero_T && (rc = do_phase_a(h, L, j))) return rc;
         if (h->sharded) {
             // sample-sharded: the region statistics of both streaming phases are summed over the ranks
-            if (!zero_T && (rc = do_exchange(h, j, 0, h->cfg.n_basis * h->cfg.dy, false))) return rc;
-            if ((rc = do_axis_update(h, j, fork_omega && ci, zero_T))) return rc;
+            if (!zero_T && (rc = do_exchange(h, L, j, 0, h->cfg.n_basis * h->cfg.dy, false))) return rc;
+            if ((rc = do_axis_update(h, L, j, ci, zero_T))) return rc;
             if (closed && j > 0) {   // replicated closed form: no samples, no exchange
-                if ((rc = do_stats_b(h, j))) return rc;
+                if ((rc = do_stats_b(h, L, j))) return rc;
                 continue;
             }
-            if ((rc = do_phase_b(h, j, false, closed ? 0 : -1))) return rc;
-            if ((rc = do_exchange(h, j, 1, h->cfg.dy + 3, false))) return rc;
-            if ((rc = do_bias_noise(h, j))) return rc;
+            if ((rc = do_phase_b(h, L, j, false, closed ? 0 : -1))) return rc;
+            if ((rc = do_exchange(h, L, j, 1, h->cfg.dy + 3, false))) return rc;
+            if ((rc = do_bias_noise(h, L, j))) return rc;
             continue;
         }
-        if ((rc = do_axis_update(h, j, fork_omega && ci, zero_T))) return rc;
+        if ((rc = do_axis_update(h, L, j, ci, zero_T))) return rc;
         if (h->dev[j].adaptive && ci) {
             // the latent functions of the next layer use the re-learnt basis (MRGP.py:632-649): statistics first,
             // then the interval search, then a second pass that only propagates
-            if ((rc = do_phase_b(h, j, true, 0))) return rc;
-            if ((rc = do_learn_intervals(h, j))) return rc;
-            if (j + 1 < J && (rc = do_phase_b(h, j, false, 1))) return rc;
+            if ((rc = do_phase_b(h, L, j, true, 0))) return rc;
+            if ((rc = do_learn_intervals(h, L, j))) return rc;
+            if (j + 1 < J && (rc = do_phase_b(h, L, j, false, 1))) return rc;
         } else if (closed && j > 0) {
             // inferred targets: statistics from the basis invariants.  In the captured sweep they follow layer 0's pass
             // on the third stream (they read the bias variances of the coarser layers, nothing of the chain waits for
             // them): k_mid1 of the next layer starts as soon as the ARD moments are there.
-            if (fork_omega && h->b0_pending) {
-                CK(cudaStreamWaitEvent(h->side2, h->ev_mid2[j], 0));   // A, cm2 of this layer (k_mid2)
-                cudaStream_t main_stream = h->stream;
-                h->stream = h->side2;
-                rc = do_stats_b(h, j);
-                h->stream = main_stream;
-                if (rc) return rc;
-            } else {
-                if ((rc = do_stats_b(h, j))) return rc;
-            }
-        } else if (closed && j == 0 && fork_omega && J > 1 && h->side2) {
+            if (b0_forked) CK(cudaStreamWaitEvent(h->side2, h->ev_mid2[j], 0));   // A, cm2 of this layer (k_mid2)
+            if ((rc = do_stats_b(h, b0_forked ? b0 : L, j))) return rc;
+        } else if (closed && j == 0 && J > 1) {
             // Layer 0's statistics pass (26 us on 147 SMs) runs on a third stream: the small-matrix chain of layer 1
             // (k_mid1 -> k_ard -> k_scale_warp on the SM left free) does not depend on it, only k_stats_b does.
-            CK(cudaEventRecord(h->ev_b0_fork, h->stream));
+            CK(cudaEventRecord(h->ev_b0_fork, L.stream));
             CK(cudaStreamWaitEvent(h->side2, h->ev_b0_fork, 0));
-            cudaStream_t main_stream = h->stream;
-            h->stream = h->side2;
-            rc = do_phase_b(h, j, true, 0);
-            h->stream = main_stream;
-            if (rc) return rc;
-            h->b0_pending = true;
+            if ((rc = do_phase_b(h, b0, j, true, 0))) return rc;
+            b0_forked = true;
         } else {
             // bias / noise update fused into the kernel tail; nothing reads the latent buffers when the layers below
             // take the closed form
-            if ((rc = do_phase_b(h, j, true, closed ? 0 : -1))) return rc;
+            if ((rc = do_phase_b(h, L, j, true, closed ? 0 : -1))) return rc;
         }
     }
-    if (fork_omega && ci) {
-        CK(cudaStreamWaitEvent(h->stream, h->ev_ard[J - 1], 0));
-        CK(cudaStreamWaitEvent(h->stream, h->ev_join[J - 1], 0));
+    if (ci) {
+        CK(cudaStreamWaitEvent(L.stream, h->ev_ard[J - 1], 0));
+        CK(cudaStreamWaitEvent(L.stream, h->ev_join[J - 1], 0));
     }
-    if (h->b0_pending) {   // join the third stream (layer 0's pass and the closed-form statistics of the other layers)
+    if (b0_forked) {   // join the third stream (layer 0's pass and the closed-form statistics of the other layers)
         CK(cudaEventRecord(h->ev_b0_done, h->side2));
-        CK(cudaStreamWaitEvent(h->stream, h->ev_b0_done, 0));
-        h->b0_pending = false;
+        CK(cudaStreamWaitEvent(L.stream, h->ev_b0_done, 0));
     }
     return MRGP_OK;
 }
@@ -1857,9 +1839,10 @@ int mrgp_build_basis(mrgp_handle *h, int32_t layer, double interval_factor, cons
         if (L_host) return fail(h, MRGP_EINVAL, "given intervals are not supported on a sharded handle");
         int rs;
         if ((rs = mrgp_build_basis_stage(h, layer, -1, interval_factor))) return rs;   // local max|x| partials
-        if ((rs = do_exchange(h, layer, 0, 1, true))) return rs;
+        const Launch L{h->stream, &h->launches};
+        if ((rs = do_exchange(h, L, layer, 0, 1, true))) return rs;
         if ((rs = mrgp_build_basis_stage(h, layer, -2, interval_factor))) return rs;   // L, lambda, S; local sum phi^2 partials
-        if ((rs = do_exchange(h, layer, 1, h->cfg.n_basis, false))) return rs;
+        if ((rs = do_exchange(h, L, layer, 1, h->cfg.n_basis, false))) return rs;
         return mrgp_build_basis_stage(h, layer, 2, interval_factor);
     }
     LayerDev &d = h->dev[layer];
@@ -1873,18 +1856,18 @@ int mrgp_build_basis(mrgp_handle *h, int32_t layer, double interval_factor, cons
     } else {
         k_absmax<<<h->n_ctas, kThreads, 0, h->stream>>>(sa);
         CK(cudaGetLastError());
-        count(h);
+        h->launches += 1;
     }
     k_region_setup<<<(lp.R + 7) / 8, 256, 0, h->stream>>>(ra);
     CK(cudaGetLastError());
-    count(h);
+    h->launches += 1;
     cudaError_t e = cudaErrorInvalidValue;
-    DISPATCH_M(h->cfg.n_basis, e = launch_phi2sum<MM>(h, sa));
+    DISPATCH_M(h->cfg.n_basis, e = launch_phi2sum<MM>(h, h->stream, sa));
     CK(e);
-    count(h);
+    h->launches += 1;
     k_reduce_d<<<lp.R, 64, 0, h->stream>>>(ra);
     CK(cudaGetLastError());
-    count(h);
+    h->launches += 1;
     d.basis_built = true;
     for (int jj = layer; jj < h->cfg.n_layers; ++jj) h->dev[jj].inv_built = false;   // s, G of the layer; D of the finer ones
     h->ystats_valid = false;
@@ -1916,7 +1899,7 @@ int mrgp_init_state(mrgp_handle *h, double noise_var0, double ard_prior_influenc
         const int total = h->plan[j].R * M;
         k_init_layer<2><<<(total + 127) / 128, 128, 0, h->stream>>>(a, j == 0 ? noise_var0 : 1.0, ard_prior_influence, logc0, rho0[0]);
         CK(cudaGetLastError());
-        count(h);
+        h->launches += 1;
     }
     {
         RegionArgs a = region_args(h, 0);
@@ -1927,7 +1910,7 @@ int mrgp_init_state(mrgp_handle *h, double noise_var0, double ard_prior_influenc
         a.ardShape = s.ardShape; a.ardScale = s.ardScale; a.ardMean = s.ardMean; a.ardLogMean = s.ardLogMean;
         k_init_shared<2><<<1, 256, 0, h->stream>>>(a, s.priorB, s.priorLogC, s.priorShape, s.priorScale, ard_prior_influence, logc0, rho0[0]);
         CK(cudaGetLastError());
-        count(h);
+        h->launches += 1;
     }
     CK(cudaMemsetAsync(h->g, 0, (size_t)(h->hi - h->lo) * h->cfg.dy * sizeof(double), h->stream));
     CK(cudaMemsetAsync(h->hvar, 0, (size_t)(h->hi - h->lo) * sizeof(double), h->stream));
@@ -1973,7 +1956,7 @@ int mrgp_get_state(mrgp_handle *h, int32_t layer, int32_t field, double *dst_hos
             ea.single_region = 0;
             k_eval_layers<2><<<(unsigned)((N + 127) / 128), 128, 0, h->stream>>>(ea);
             CK(cudaGetLastError());
-            count(h);
+            h->launches += 1;
         }
     }
     CK(cudaMemcpyAsync(dst_host, f.ptr, (size_t)f.n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
@@ -2001,26 +1984,26 @@ int mrgp_set_state(mrgp_handle *h, int32_t layer, int32_t field, const double *s
 int mrgp_phase_a(mrgp_handle *h, int32_t layer) {
     if (h) h->stream_ops += 1;
     int rc = check_ready(h, layer, true);
-    return rc ? rc : do_phase_a(h, layer);
+    return rc ? rc : do_phase_a(h, Launch{h->stream, &h->launches}, layer);
 }
 
 int mrgp_axis_update(mrgp_handle *h, int32_t layer) {
     if (h) h->stream_ops += 1;
     int rc = check_ready(h, layer, true);
-    return rc ? rc : do_axis_update(h, layer, false);
+    return rc ? rc : do_axis_update(h, Launch{h->stream, &h->launches}, layer, false);
 }
 
 int mrgp_phase_b(mrgp_handle *h, int32_t layer) {
     if (h) h->stream_ops += 1;
     int rc = check_ready(h, layer, true);
-    return rc ? rc : do_phase_b(h, layer, false);
+    return rc ? rc : do_phase_b(h, Launch{h->stream, &h->launches}, layer, false);
 }
 
 int mrgp_bias_noise(mrgp_handle *h, int32_t layer) {
     if (h) h->stream_ops += 1;
     int rc = check_ready(h, layer, true);
     if (!rc && layer == h->cfg.n_layers - 1) h->sweeps_done += 1;
-    return rc ? rc : do_bias_noise(h, layer);
+    return rc ? rc : do_bias_noise(h, Launch{h->stream, &h->launches}, layer);
 }
 
 int mrgp_set_adaptive_intervals(mrgp_handle *h, int32_t layer, int32_t enabled, int32_t use_prior, double factor_lo, double factor_hi) {
@@ -2048,7 +2031,7 @@ int mrgp_learn_intervals(mrgp_handle *h, int32_t layer) {
     int rc = check_ready(h, layer, true);
     if (rc) return rc;
     if (!h->dev[layer].adaptive) return fail(h, MRGP_ESTATE, "adaptive intervals are not enabled on this layer");
-    return do_learn_intervals(h, layer);
+    return do_learn_intervals(h, Launch{h->stream, &h->launches}, layer);
 }
 
 int mrgp_interval_failures(mrgp_handle *h, uint64_t *out) {
@@ -2067,9 +2050,10 @@ int mrgp_refresh_statistics(mrgp_handle *h) {
     h->stream_ops += 1;
     if ((rc = adopt_prefetched(h))) return rc;
     if (!use_fused(h)) return MRGP_OK;   // the multi-kernel sweep streams layer 0: nothing to prepare
-    if ((rc = build_invariants(h))) return rc;
+    const Launch L{h->stream, &h->launches};
+    if ((rc = build_invariants(h, L))) return rc;
     if (!h->chain_uploaded && (rc = upload_chain_model(h))) return rc;
-    return do_ystats(h);
+    return do_ystats(h, L);
 }
 
 int mrgp_sweep(mrgp_handle *h, int32_t n_iter) {
@@ -2080,30 +2064,26 @@ int mrgp_sweep(mrgp_handle *h, int32_t n_iter) {
     if (h->sharded && !h->comm.ready)
         return fail(h, MRGP_ESTATE, "mrgp_sweep on a sharded handle needs the peer exchange (mrgp_comm_bind); without it drive the phases and the all-reduces from the host");
     const bool fused = use_fused(h);
+    const Launch L{h->stream, &h->launches};
     if (fused) {
-        if ((rc = build_invariants(h))) return rc;
+        if ((rc = build_invariants(h, L))) return rc;
         if (!h->chain_uploaded && (rc = upload_chain_model(h))) return rc;
-        if (!h->ystats_valid && (rc = do_ystats(h))) return rc;
+        if (!h->ystats_valid && (rc = do_ystats(h, L))) return rc;
     }
     if (fused && h->direct_launch) {
         for (int it = 0; it < n_iter; ++it)
-            if ((rc = sweep_once(h, true))) return rc;   // count() adds the launches (not capturing)
+            if ((rc = sweep_once(h, L))) return rc;
         h->sweeps_done += n_iter;
         return MRGP_OK;
     }
     if (!h->graph_exec) {
-        if ((rc = build_invariants(h))) return rc;
+        if ((rc = build_invariants(h, L))) return rc;
         h->launches_per_sweep = 0;
-        h->capturing = true;
         cudaError_t e = cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal);
-        if (e != cudaSuccess) {
-            h->capturing = false;
-            return fail(h, MRGP_ECUDA, "cudaStreamBeginCapture: %s", cudaGetErrorString(e));
-        }
-        rc = sweep_once(h, true);
+        if (e != cudaSuccess) return fail(h, MRGP_ECUDA, "cudaStreamBeginCapture: %s", cudaGetErrorString(e));
+        rc = sweep_once(h, Launch{h->stream, &h->launches_per_sweep});
         cudaGraph_t graph = nullptr;
         e = cudaStreamEndCapture(h->stream, &graph);
-        h->capturing = false;
         if (rc) {
             if (graph) cudaGraphDestroy(graph);
             return rc;
@@ -2177,7 +2157,7 @@ static int group_prepare(mrgp_group *g) {
             g->error = h->err;
             return rc;
         }
-        if ((rc = build_invariants(h))) return rc;
+        if ((rc = build_invariants(h, Launch{h->stream, &h->launches}))) return rc;
         const bool f = use_fused(h) && ystats_small(h);
         batched = batched && f && chain_solver_size(h->cfg.n_basis) == chain_solver_size(g->handles[0]->cfg.n_basis) &&
                   chain_cluster_size(h) == chain_cluster_size(g->handles[0]);
@@ -2217,7 +2197,7 @@ static int group_prepare(mrgp_group *g) {
     };
     for (int i = 0; i < n && rc == MRGP_OK; ++i) {
         mrgp_handle *h = g->handles[i];
-        if (use_fused(h) && !h->ystats_valid && (rc = do_ystats(h))) break;
+        if (use_fused(h) && !h->ystats_valid && (rc = do_ystats(h, Launch{h->stream, &h->launches}))) break;
         if (cudaStreamSynchronize(h->stream) != cudaSuccess) rc = MRGP_ECUDA;
         if (cudaStreamCreateWithFlags(&tmp[i], cudaStreamNonBlocking) != cudaSuccess ||
             cudaEventCreateWithFlags(&done[i], cudaEventDisableTiming) != cudaSuccess)
@@ -2231,16 +2211,8 @@ static int group_prepare(mrgp_group *g) {
         for (int i = 0; i < n; ++i) {
             mrgp_handle *h = g->handles[i];
             cudaStreamWaitEvent(tmp[i], start, 0);
-            cudaStream_t saved = h->stream;
-            h->stream = tmp[i];
-            const int64_t saved_lps = h->launches_per_sweep;
-            h->launches_per_sweep = 0;
-            h->capturing = true;
-            const int r = sweep_once(h, true);
-            h->capturing = false;
-            h->stream = saved;
-            g->launches_per_sweep[i] = h->launches_per_sweep;
-            h->launches_per_sweep = saved_lps;
+            g->launches_per_sweep[i] = 0;
+            const int r = sweep_once(h, Launch{tmp[i], &g->launches_per_sweep[i]});
             if (r && rc == MRGP_OK) rc = r;
             cudaEventRecord(done[i], tmp[i]);
             cudaStreamWaitEvent(g->stream, done[i], 0);
@@ -2392,7 +2364,7 @@ int mrgp_elbo(mrgp_handle *h, double *out_host) {
     }
     k_elbo<2><<<dim3((unsigned)h->cfg.n_layers, (unsigned)h->elbo_chunks), 256, 0, h->stream>>>(h->elbo_args, h->elbo_out, h->elbo_part, h->elbo_counter);
     CK(cudaGetLastError());
-    count(h);
+    h->launches += 1;
     CK(cudaMemcpyAsync(out_host, h->elbo_out, (size_t)h->cfg.n_layers * 6 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     if (h->elbo_no_sync) return MRGP_OK;
     CK(cudaStreamSynchronize(h->stream));
@@ -2464,7 +2436,7 @@ int mrgp_predict_mean(mrgp_handle *h, const double *x_test_dev, int64_t n_test, 
     ea.out_var = nullptr;
     k_eval_layers<2><<<(unsigned)((n_test + 127) / 128), 128, 0, h->stream>>>(ea);
     CK(cudaGetLastError());
-    count(h);
+    h->launches += 1;
     CK(cudaStreamSynchronize(h->stream));
     return MRGP_OK;
 }
@@ -2494,7 +2466,7 @@ int mrgp_predict_var_indexed(mrgp_handle *h, const double *x_test_dev, int64_t n
     ea.out_var = out_dev;
     k_eval_var_indexed<2><<<(unsigned)((n_test + 127) / 128), 128, 0, h->stream>>>(ea);
     CK(cudaGetLastError());
-    count(h);
+    h->launches += 1;
     CK(cudaStreamSynchronize(h->stream));
     return MRGP_OK;
 }
@@ -2512,7 +2484,7 @@ int mrgp_predict_var(mrgp_handle *h, const double *x_test_dev, int64_t n_test, d
     ea.out_var = out_dev;
     k_eval_layers<2><<<(unsigned)((n_test + 127) / 128), 128, 0, h->stream>>>(ea);
     CK(cudaGetLastError());
-    count(h);
+    h->launches += 1;
     CK(cudaStreamSynchronize(h->stream));
     return MRGP_OK;
 }
@@ -2624,7 +2596,7 @@ int mrgp_exchange(mrgp_handle *h, int32_t layer, int32_t which) {
     if (rc) return rc;
     if (!h->sharded) return fail(h, MRGP_ESTATE, "not a sharded handle");
     if (which != MRGP_X_PHASE_A && which != MRGP_X_PHASE_B) return fail(h, MRGP_EINVAL, "which must be MRGP_X_PHASE_A or MRGP_X_PHASE_B");
-    return do_exchange(h, layer, which, which == MRGP_X_PHASE_A ? h->cfg.n_basis * h->cfg.dy : h->cfg.dy + 3, false);
+    return do_exchange(h, Launch{h->stream, &h->launches}, layer, which, which == MRGP_X_PHASE_A ? h->cfg.n_basis * h->cfg.dy : h->cfg.dy + 3, false);
 }
 
 int mrgp_region_sums(mrgp_handle *h, int32_t layer, int32_t which) {
@@ -2636,7 +2608,7 @@ int mrgp_region_sums(mrgp_handle *h, int32_t layer, int32_t which) {
     const int total = lp.R * h->part_stride;
     k_region_sums<false><<<(total + 255) / 256, 256, 0, h->stream>>>(h->dev[layer].region_run, h->part, h->part_stride, nv, lp.R, h->xchg);
     CK(cudaGetLastError());
-    count(h);
+    h->launches += 1;
     return MRGP_OK;
 }
 
@@ -2662,33 +2634,33 @@ int mrgp_build_basis_stage(mrgp_handle *h, int32_t layer, int32_t stage, double 
     if (stage == -1) {         // peer exchange variant of stage 0: partials only
         k_absmax<<<h->n_ctas, kThreads, 0, h->stream>>>(sa);
         CK(cudaGetLastError());
-        count(h);
+        h->launches += 1;
     } else if (stage == -2) {  // peer exchange variant of stage 1
         k_region_setup<<<(lp.R + 7) / 8, 256, 0, h->stream>>>(ra);
         CK(cudaGetLastError());
         cudaError_t e = cudaErrorInvalidValue;
-        DISPATCH_M(h->cfg.n_basis, e = launch_phi2sum<MM>(h, sa));
+        DISPATCH_M(h->cfg.n_basis, e = launch_phi2sum<MM>(h, h->stream, sa));
         CK(e);
-        count(h, 2);
+        h->launches += 2;
     } else if (stage == 0) {   // local max|x| per region -> exchange buffer (caller: all-reduce MAX)
         k_absmax<<<h->n_ctas, kThreads, 0, h->stream>>>(sa);
         CK(cudaGetLastError());
         k_region_sums<true><<<(total + 255) / 256, 256, 0, h->stream>>>(d.region_run, h->part, h->part_stride, 1, lp.R, h->xchg);
         CK(cudaGetLastError());
-        count(h, 2);
+        h->launches += 2;
     } else if (stage == 1) {   // L, lambda, S from the global max; local sum phi^2 -> exchange buffer (all-reduce SUM)
         k_region_setup<<<(lp.R + 7) / 8, 256, 0, h->stream>>>(ra);
         CK(cudaGetLastError());
         cudaError_t e = cudaErrorInvalidValue;
-        DISPATCH_M(h->cfg.n_basis, e = launch_phi2sum<MM>(h, sa));
+        DISPATCH_M(h->cfg.n_basis, e = launch_phi2sum<MM>(h, h->stream, sa));
         CK(e);
         k_region_sums<false><<<(total + 255) / 256, 256, 0, h->stream>>>(d.region_run, h->part, h->part_stride, h->cfg.n_basis, lp.R, h->xchg);
         CK(cudaGetLastError());
-        count(h, 3);
+        h->launches += 3;
     } else if (stage == 2) {   // d = global sum phi^2
         k_reduce_d<<<lp.R, 64, 0, h->stream>>>(ra);
         CK(cudaGetLastError());
-        count(h);
+        h->launches += 1;
         d.basis_built = true;
         for (int jj = layer; jj < h->cfg.n_layers; ++jj) h->dev[jj].inv_built = false;   // s, G of the layer; D of the finer ones
         h->ystats_valid = false;
