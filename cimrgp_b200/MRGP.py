@@ -155,7 +155,8 @@ class MultiResolutionGaussianProcess(object):
             engine_kw.update(_engine_opts)      # shared stream / workspace slice / pinned staging (cimrgp_b200/batch.py)
         if distributed:
             # one process per GPU (torch.distributed initialised by the caller): this rank keeps its chunk of
-            # the samples, the region statistics are all-reduced, the model state is replicated on every rank
+            # the samples, the region statistics are summed over the ranks by the peer exchange, the model state is
+            # replicated on every rank
             import torch.distributed as dist
             from .distributed import ShardedEngine
             self._engine = ShardedEngine(x_used, y_train, self._offsets, n_basis, dist.get_rank(),

@@ -9,7 +9,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'libcimrgp.so')
 
 COMM_BLOB_BYTES = 128
-ABI_VERSION = 4
+ABI_VERSION = 5
 MODE_CI, MODE_FI = 0, 1
 OK, EINVAL, ENODEVICE, ECUDA, ESTATE, ENOMEM = 0, -1, -2, -3, -4, -5
 
@@ -89,9 +89,6 @@ SIGNATURES = {
     'mrgp_comm_bind': (C.c_int, [_P, C.c_int32, C.c_int32, C.c_void_p, C.POINTER(C.c_int64)]),
     'mrgp_exchange': (C.c_int, [_P, C.c_int32, C.c_int32]),
     'mrgp_set_all_inputs_host': (C.c_int, [_P, _D]),
-    'mrgp_region_sums': (C.c_int, [_P, C.c_int32, C.c_int32]),
-    'mrgp_exchange_buffer': (C.c_int, [_P, C.c_int32, C.c_int32, C.POINTER(_P), C.POINTER(C.c_size_t)]),
-    'mrgp_build_basis_stage': (C.c_int, [_P, C.c_int32, C.c_int32, C.c_double]),
     'mrgp_launch_count': (C.c_int64, [_P]),
     'mrgp_cholesky_count': (C.c_int64, [_P]),
     'mrgp_batched_cholesky': (C.c_int, [_P, _P, C.c_int32, C.c_int64, _P]),

@@ -873,13 +873,13 @@ int do_bias_noise(mrgp_handle *h, const Launch &L, int j) {
     return do_bias_noise_shared(h, L, j);
 }
 
-// One exchange over peer memory: local dense sums -> arena slot, publish, reduce over the owning ranks -> h->xchg.
-int do_exchange(mrgp_handle *h, const Launch &L, int j, int slot, int nv, bool is_max) {
+// One exchange over peer memory: local dense sums -> arena slot (picked on the device from the exchange number),
+// publish, reduce over the owning ranks -> h->xchg.
+int do_exchange(mrgp_handle *h, const Launch &L, int j, int nv, bool is_max) {
     if (!h->comm.ready) return fail(h, MRGP_ESTATE, "no peer exchange bound: mrgp_comm_export / mrgp_comm_bind first");
     const LayerPlan &lp = h->plan[j];
     LayerDev &d = h->dev[j];
     const int total = lp.R * h->part_stride;
-    (void)slot;   // the arena slot follows the exchange number on the device (k_comm_sums_signal)
     if (h->part_stride > 256) return fail(h, MRGP_EINVAL, "exchange rows of more than 256 values are not supported");
     if (is_max)
         k_comm_sums_signal<true><<<lp.R, 256, 0, L.stream>>>(h->comm.args, d.region_run, h->part, h->part_stride, nv, h->comm.arena, h->comm.counter);
@@ -1140,7 +1140,7 @@ int do_ystats(mrgp_handle *h, const Launch &L) {
         const int32_t *rr = d.region_run;
         const double *part = h->part;
         if (h->sharded) {   // sum the statistics of the ranks' chunks
-            int rc = do_exchange(h, L, 0, 0, padded_basis(M) * DY + DY + 1, false);
+            int rc = do_exchange(h, L, 0, padded_basis(M) * DY + DY + 1, false);
             if (rc) return rc;
             rr = d.ident_run;
             part = h->xchg;
@@ -1259,14 +1259,14 @@ int sweep_once(mrgp_handle *h, const Launch &L) {
         if (!zero_T && (rc = do_phase_a(h, L, j))) return rc;
         if (h->sharded) {
             // sample-sharded: the region statistics of both streaming phases are summed over the ranks
-            if (!zero_T && (rc = do_exchange(h, L, j, 0, h->cfg.n_basis * h->cfg.dy, false))) return rc;
+            if (!zero_T && (rc = do_exchange(h, L, j, h->cfg.n_basis * h->cfg.dy, false))) return rc;
             if ((rc = do_axis_update(h, L, j, ci, zero_T))) return rc;
             if (closed && j > 0) {   // replicated closed form: no samples, no exchange
                 if ((rc = do_stats_b(h, L, j))) return rc;
                 continue;
             }
             if ((rc = do_phase_b(h, L, j, false, closed ? 0 : -1))) return rc;
-            if ((rc = do_exchange(h, L, j, 1, h->cfg.dy + 3, false))) return rc;
+            if ((rc = do_exchange(h, L, j, h->cfg.dy + 3, false))) return rc;
             if ((rc = do_bias_noise(h, L, j))) return rc;
             continue;
         }
@@ -1828,25 +1828,15 @@ int mrgp_set_spectral(mrgp_handle *h, int32_t layer, int32_t use_prior, double n
     return MRGP_OK;
 }
 
-int mrgp_build_basis_stage(mrgp_handle *h, int32_t layer, int32_t stage, double interval_factor);
-
 int mrgp_build_basis(mrgp_handle *h, int32_t layer, double interval_factor, const double *L_host) {
     if (h) h->stream_ops += 1;
     int rc = check_ready(h, layer, false);
     if (rc) return rc;
-    if (h->sharded && !h->comm.ready) return fail(h, MRGP_ESTATE, "sharded handle: bind the peer exchange first, or use mrgp_build_basis_stage with all-reduces in between");
-    if (h->sharded) {
-        if (L_host) return fail(h, MRGP_EINVAL, "given intervals are not supported on a sharded handle");
-        int rs;
-        if ((rs = mrgp_build_basis_stage(h, layer, -1, interval_factor))) return rs;   // local max|x| partials
-        const Launch L{h->stream, &h->launches};
-        if ((rs = do_exchange(h, L, layer, 0, 1, true))) return rs;
-        if ((rs = mrgp_build_basis_stage(h, layer, -2, interval_factor))) return rs;   // L, lambda, S; local sum phi^2 partials
-        if ((rs = do_exchange(h, L, layer, 1, h->cfg.n_basis, false))) return rs;
-        return mrgp_build_basis_stage(h, layer, 2, interval_factor);
-    }
+    if (h->sharded && !h->comm.ready) return fail(h, MRGP_ESTATE, "sharded handle: bind the peer exchange first (mrgp_comm_export / mrgp_comm_bind)");
+    if (h->sharded && L_host) return fail(h, MRGP_EINVAL, "given intervals are not supported on a sharded handle");
     LayerDev &d = h->dev[layer];
     const LayerPlan &lp = h->plan[layer];
+    const Launch L{h->stream, &h->launches};
     StreamArgs sa = stream_args(h, layer);
     RegionArgs ra = region_args(h, layer);
     ra.interval_factor = interval_factor;
@@ -1858,6 +1848,8 @@ int mrgp_build_basis(mrgp_handle *h, int32_t layer, double interval_factor, cons
         CK(cudaGetLastError());
         h->launches += 1;
     }
+    // sharded: L, lambda, S from the max|x| of the region over all ranks, d from the sum of phi^2 over all ranks
+    if (h->sharded && (rc = do_exchange(h, L, layer, 1, true))) return rc;
     k_region_setup<<<(lp.R + 7) / 8, 256, 0, h->stream>>>(ra);
     CK(cudaGetLastError());
     h->launches += 1;
@@ -1865,6 +1857,7 @@ int mrgp_build_basis(mrgp_handle *h, int32_t layer, double interval_factor, cons
     DISPATCH_M(h->cfg.n_basis, e = launch_phi2sum<MM>(h, h->stream, sa));
     CK(e);
     h->launches += 1;
+    if (h->sharded && (rc = do_exchange(h, L, layer, h->cfg.n_basis, false))) return rc;
     k_reduce_d<<<lp.R, 64, 0, h->stream>>>(ra);
     CK(cudaGetLastError());
     h->launches += 1;
@@ -2062,7 +2055,7 @@ int mrgp_sweep(mrgp_handle *h, int32_t n_iter) {
     if (rc) return rc;
     if (n_iter < 0) return fail(h, MRGP_EINVAL, "n_iter < 0");
     if (h->sharded && !h->comm.ready)
-        return fail(h, MRGP_ESTATE, "mrgp_sweep on a sharded handle needs the peer exchange (mrgp_comm_bind); without it drive the phases and the all-reduces from the host");
+        return fail(h, MRGP_ESTATE, "mrgp_sweep on a sharded handle needs the peer exchange (mrgp_comm_export / mrgp_comm_bind)");
     const bool fused = use_fused(h);
     const Launch L{h->stream, &h->launches};
     if (fused) {
@@ -2578,8 +2571,6 @@ int mrgp_comm_bind(mrgp_handle *h, int32_t rank, int32_t world, const void *blob
         a.arena[q] = reinterpret_cast<const double *>(static_cast<char *>(base) + 512);
     }
     // same shared-memory carveout as the rest of the sweep: no SM reconfiguration around the exchanges
-    CK(cudaFuncSetAttribute(k_region_sums<false>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    CK(cudaFuncSetAttribute(k_region_sums<true>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
     CK(cudaFuncSetAttribute(k_comm_sums_signal<false>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
     CK(cudaFuncSetAttribute(k_comm_sums_signal<true>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
     CK(cudaFuncSetAttribute(k_comm_reduce<false>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
@@ -2596,79 +2587,7 @@ int mrgp_exchange(mrgp_handle *h, int32_t layer, int32_t which) {
     if (rc) return rc;
     if (!h->sharded) return fail(h, MRGP_ESTATE, "not a sharded handle");
     if (which != MRGP_X_PHASE_A && which != MRGP_X_PHASE_B) return fail(h, MRGP_EINVAL, "which must be MRGP_X_PHASE_A or MRGP_X_PHASE_B");
-    return do_exchange(h, Launch{h->stream, &h->launches}, layer, which, which == MRGP_X_PHASE_A ? h->cfg.n_basis * h->cfg.dy : h->cfg.dy + 3, false);
-}
-
-int mrgp_region_sums(mrgp_handle *h, int32_t layer, int32_t which) {
-    int rc = check_ready(h, layer, false);
-    if (rc) return rc;
-    if (!h->sharded) return fail(h, MRGP_ESTATE, "not a sharded handle");
-    const LayerPlan &lp = h->plan[layer];
-    const int nv = which == MRGP_X_PHASE_A ? h->cfg.n_basis * h->cfg.dy : h->cfg.dy + 3;
-    const int total = lp.R * h->part_stride;
-    k_region_sums<false><<<(total + 255) / 256, 256, 0, h->stream>>>(h->dev[layer].region_run, h->part, h->part_stride, nv, lp.R, h->xchg);
-    CK(cudaGetLastError());
-    h->launches += 1;
-    return MRGP_OK;
-}
-
-int mrgp_exchange_buffer(mrgp_handle *h, int32_t layer, int32_t which, void **dev_ptr, size_t *n_doubles) {
-    if (!h || !dev_ptr || !n_doubles || layer < 0 || layer >= h->cfg.n_layers) return fail(h, MRGP_EINVAL, "bad argument");
-    if (!h->bound) return fail(h, MRGP_ESTATE, "no workspace bound");
-    (void)which;
-    *dev_ptr = h->xchg;
-    *n_doubles = (size_t)h->plan[layer].R * h->part_stride;
-    return MRGP_OK;
-}
-
-int mrgp_build_basis_stage(mrgp_handle *h, int32_t layer, int32_t stage, double interval_factor) {
-    int rc = check_ready(h, layer, false);
-    if (rc) return rc;
-    if (!h->sharded) return fail(h, MRGP_ESTATE, "not a sharded handle");
-    LayerDev &d = h->dev[layer];
-    const LayerPlan &lp = h->plan[layer];
-    StreamArgs sa = stream_args(h, layer);
-    RegionArgs ra = region_args(h, layer);
-    ra.interval_factor = interval_factor;
-    const int total = lp.R * h->part_stride;
-    if (stage == -1) {         // peer exchange variant of stage 0: partials only
-        k_absmax<<<h->n_ctas, kThreads, 0, h->stream>>>(sa);
-        CK(cudaGetLastError());
-        h->launches += 1;
-    } else if (stage == -2) {  // peer exchange variant of stage 1
-        k_region_setup<<<(lp.R + 7) / 8, 256, 0, h->stream>>>(ra);
-        CK(cudaGetLastError());
-        cudaError_t e = cudaErrorInvalidValue;
-        DISPATCH_M(h->cfg.n_basis, e = launch_phi2sum<MM>(h, h->stream, sa));
-        CK(e);
-        h->launches += 2;
-    } else if (stage == 0) {   // local max|x| per region -> exchange buffer (caller: all-reduce MAX)
-        k_absmax<<<h->n_ctas, kThreads, 0, h->stream>>>(sa);
-        CK(cudaGetLastError());
-        k_region_sums<true><<<(total + 255) / 256, 256, 0, h->stream>>>(d.region_run, h->part, h->part_stride, 1, lp.R, h->xchg);
-        CK(cudaGetLastError());
-        h->launches += 2;
-    } else if (stage == 1) {   // L, lambda, S from the global max; local sum phi^2 -> exchange buffer (all-reduce SUM)
-        k_region_setup<<<(lp.R + 7) / 8, 256, 0, h->stream>>>(ra);
-        CK(cudaGetLastError());
-        cudaError_t e = cudaErrorInvalidValue;
-        DISPATCH_M(h->cfg.n_basis, e = launch_phi2sum<MM>(h, h->stream, sa));
-        CK(e);
-        k_region_sums<false><<<(total + 255) / 256, 256, 0, h->stream>>>(d.region_run, h->part, h->part_stride, h->cfg.n_basis, lp.R, h->xchg);
-        CK(cudaGetLastError());
-        h->launches += 3;
-    } else if (stage == 2) {   // d = global sum phi^2
-        k_reduce_d<<<lp.R, 64, 0, h->stream>>>(ra);
-        CK(cudaGetLastError());
-        h->launches += 1;
-        d.basis_built = true;
-        for (int jj = layer; jj < h->cfg.n_layers; ++jj) h->dev[jj].inv_built = false;   // s, G of the layer; D of the finer ones
-        h->ystats_valid = false;
-        drop_graph(h);
-    } else {
-        return fail(h, MRGP_EINVAL, "stage must be 0, 1 or 2");
-    }
-    return MRGP_OK;
+    return do_exchange(h, Launch{h->stream, &h->launches}, layer, which == MRGP_X_PHASE_A ? h->cfg.n_basis * h->cfg.dy : h->cfg.dy + 3, false);
 }
 
 int64_t mrgp_launch_count(const mrgp_handle *h) { return h ? h->launches : -1; }

@@ -1552,22 +1552,6 @@ __global__ void __launch_bounds__(kOmegaThreads) k_scale(RegionArgs a) {
     ts_end(a.ts, a.layer * 4 + 3);
 }
 
-// Dense per-region sums of the run partials (multi-GPU exchange buffer, SURVEY.md §8e): out[r][v] = sum over the
-// local runs of region r (zero for regions without local samples); MAX = true for the max|x| partials.
-template <bool MAX>
-__global__ void k_region_sums(const int32_t *region_run, const double *part, int part_stride, int nv, int R, double *out) {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= R * part_stride) return;
-    const int r = t / part_stride, v = t % part_stride;
-    double acc = 0.0;
-    if (v < nv)
-        for (int q = region_run[r]; q < region_run[r + 1]; ++q) {
-            const double x = part[(size_t)q * part_stride + v];
-            acc = MAX ? fmax(acc, x) : acc + x;
-        }
-    out[(size_t)r * part_stride + v] = acc;   // padding columns are kept at zero
-}
-
 // The same solve for M <= 32 in ONE warp, matrices resident in registers: lane i owns row i of the kernel table
 // (and of the Newton matrix), every loop over the M columns is unrolled, the only communication is warp
 // shuffles plus two transposes through shared memory per Newton step.  No block barriers: a Newton step costs

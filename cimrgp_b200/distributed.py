@@ -5,11 +5,9 @@ streaming phase the per-region sufficient statistics (<= R x 60 doubles per laye
 and the small-matrix steps are replicated (identical inputs -> identical state on every rank, no broadcast).
 SURVEY.md §8e.
 
-exchange='peer' (default): the library's own exchange over peer memory (NVLink / NVSwitch): torch.distributed is
-used once, to all-gather the 128-byte arena descriptions; afterwards a sweep is one CUDA graph of the library's
-kernels, exchanges included (include/cimrgp.h, "sample sharding").
-exchange='nccl': the comparison arm - one NCCL all-reduce per phase through torch.distributed, the sequence
-captured in a torch CUDA graph.
+The sums go through the library's own exchange over peer memory (NVLink / NVSwitch): torch.distributed is used
+once, to all-gather the 128-byte arena descriptions, and at the barrier of close(); a sweep is one CUDA graph of
+the library's kernels, exchanges included (include/cimrgp.h, "sample sharding").
 """
 import ctypes as C
 
@@ -29,15 +27,11 @@ def chunk_bounds(n_samples, world_size, rank):
 
 
 class TorchComm(object):
-    """all-reduce of a device tensor over a torch.distributed process group (NCCL on GPUs)."""
+    """All-gather and barrier over a torch.distributed process group."""
 
     def __init__(self, group=None):
         import torch.distributed as dist
         self.dist, self.group = dist, group
-
-    def all_reduce(self, tensor, op):
-        d = self.dist
-        d.all_reduce(tensor, op=d.ReduceOp.MAX if op == 'max' else d.ReduceOp.SUM, group=self.group)
 
     def all_gather_bytes(self, payload):
         out = [None] * self.dist.get_world_size(self.group)
@@ -49,13 +43,9 @@ class TorchComm(object):
 
 
 class ShardedEngine(Engine):
-    def __init__(self, x_norm, y, offsets, n_basis, rank, world_size, comm=None, exchange=None, **kw):
-        import os
+    def __init__(self, x_norm, y, offsets, n_basis, rank, world_size, comm=None, **kw):
         self.comm = comm if comm is not None else TorchComm()
         self.rank, self.world_size = rank, world_size
-        self.exchange = exchange if exchange is not None else os.environ.get('MRGP_EXCHANGE', 'peer')
-        if self.exchange not in ('peer', 'nccl'):
-            raise ValueError("exchange must be 'peer' or 'nccl'")
         n_total = int(offsets[0][-1])
         # the same deterministic check on every rank, BEFORE any collective: either all ranks raise or none does
         empty = [q for q in range(world_size) if chunk_bounds(n_total, world_size, q)[1] <= chunk_bounds(n_total, world_size, q)[0]]
@@ -64,45 +54,27 @@ class ShardedEngine(Engine):
                              'most %d ranks' % (n_total, world_size, empty, max(1, -(-n_total // 32))))
         lo, hi = chunk_bounds(n_total, world_size, rank)
         Engine.__init__(self, x_norm[lo:hi], y[lo:hi], offsets, n_basis, chunk=(lo, hi), defer_build=True, **kw)
-        torch = self.torch
-        self._graph, self._xchg = None, []
-        if self.exchange == 'peer':
-            blob = C.create_string_buffer(_lib.COMM_BLOB_BYTES)
-            self._ck(self.lib.mrgp_comm_export(self.handle, blob))
-            blobs = b''.join(self.comm.all_gather_bytes(blob.raw))
-            bounds = (C.c_int64 * (world_size + 1))(*([chunk_bounds(n_total, world_size, q)[0] for q in range(world_size)]
-                                                      + [n_total]))
-            self._ck(self.lib.mrgp_comm_bind(self.handle, rank, world_size, blobs, bounds))
-            if self.mode == 'ci' and self.J > 1:
-                # inputs of all ranks (x only, 8 B per sample): the closed-form statistics of the upper layers
-                xa = np.ascontiguousarray(x_norm, dtype=np.float64)
-                self._ck(self.lib.mrgp_set_all_inputs_host(self.handle, _lib._dptr(xa) if hasattr(_lib, '_dptr') else
-                                                           xa.ctypes.data_as(C.POINTER(C.c_double))))
-                self.synchronize()
-            for j in range(self.J):
-                self._ck(self.lib.mrgp_build_basis(self.handle, j, float(self._interval_factor[j]), None))
-            self._ck(self.lib.mrgp_init_state(self.handle, *self._init_args))
+        blob = C.create_string_buffer(_lib.COMM_BLOB_BYTES)
+        self._ck(self.lib.mrgp_comm_export(self.handle, blob))
+        blobs = b''.join(self.comm.all_gather_bytes(blob.raw))
+        bounds = (C.c_int64 * (world_size + 1))(*([chunk_bounds(n_total, world_size, q)[0] for q in range(world_size)]
+                                                  + [n_total]))
+        self._ck(self.lib.mrgp_comm_bind(self.handle, rank, world_size, blobs, bounds))
+        if self.mode == 'ci' and self.J > 1:
+            # inputs of all ranks (x only, 8 B per sample): the closed-form statistics of the upper layers
+            xa = np.ascontiguousarray(x_norm, dtype=np.float64)
+            self._ck(self.lib.mrgp_set_all_inputs_host(self.handle, _lib._dptr(xa) if hasattr(_lib, '_dptr') else
+                                                       xa.ctypes.data_as(C.POINTER(C.c_double))))
             self.synchronize()
-            self.comm.sync()
-            return
         for j in range(self.J):
-            ptr, n = C.c_void_p(), C.c_size_t()
-            self._ck(self.lib.mrgp_exchange_buffer(self.handle, j, 0, C.byref(ptr), C.byref(n)))
-            off = ptr.value - self.workspace.data_ptr()
-            self._xchg.append(self.workspace[off:off + 8 * n.value].view(torch.float64))
-        with torch.cuda.stream(self.stream):
-            for j in range(self.J):
-                self._ck(self.lib.mrgp_build_basis_stage(self.handle, j, 0, float(self._interval_factor[j])))
-                self.comm.all_reduce(self._xchg[j], 'max')
-                self._ck(self.lib.mrgp_build_basis_stage(self.handle, j, 1, float(self._interval_factor[j])))
-                self.comm.all_reduce(self._xchg[j], 'sum')
-                self._ck(self.lib.mrgp_build_basis_stage(self.handle, j, 2, float(self._interval_factor[j])))
-            self._ck(self.lib.mrgp_init_state(self.handle, *self._init_args))
+            self._ck(self.lib.mrgp_build_basis(self.handle, j, float(self._interval_factor[j]), None))
+        self._ck(self.lib.mrgp_init_state(self.handle, *self._init_args))
         self.synchronize()
+        self.comm.sync()
 
     def close(self):
-        """Collective on the peer path: no rank may free its arena while a peer can still read it."""
-        if self.handle is not None and self.exchange == 'peer':
+        """Collective: no rank may free its arena while a peer can still read it."""
+        if self.handle is not None:
             try:
                 self.synchronize()
                 self.comm.sync()
@@ -120,10 +92,6 @@ class ShardedEngine(Engine):
             pass
 
     def sweep_stepwise(self):
-        if self.exchange != 'peer':
-            with self.torch.cuda.stream(self.stream):
-                self._sweep_body()
-            return
         lib, h = self.lib, self.handle
         for j in range(self.J):
             self._ck(lib.mrgp_phase_a(h, j))
@@ -133,49 +101,15 @@ class ShardedEngine(Engine):
             self._ck(lib.mrgp_exchange(h, j, 1))
             self._ck(lib.mrgp_bias_noise(h, j))
 
-    def _sweep_body(self):
-        lib, h = self.lib, self.handle
-        for j in range(self.J):
-            self._ck(lib.mrgp_phase_a(h, j))
-            self._ck(lib.mrgp_region_sums(h, j, 0))
-            self.comm.all_reduce(self._xchg[j], 'sum')
-            self._ck(lib.mrgp_axis_update(h, j))
-            self._ck(lib.mrgp_phase_b(h, j))
-            self._ck(lib.mrgp_region_sums(h, j, 1))
-            self.comm.all_reduce(self._xchg[j], 'sum')
-            self._ck(lib.mrgp_bias_noise(h, j))
-
-    def sweep(self, n_iter=1, use_graph=None):
-        import os
-        torch = self.torch
+    def sweep(self, n_iter=1, use_graph=True):
+        """n_iter sweeps: one captured CUDA graph each, or (use_graph=False) phase by phase through mrgp_exchange."""
         if n_iter <= 0:
             return
-        if self.exchange == 'peer':
-            if use_graph is False:
-                for _ in range(n_iter):
-                    self.sweep_stepwise()
-            else:
-                self._ck(self.lib.mrgp_sweep(self.handle, int(n_iter)))
-            return
-        if use_graph is None:
-            use_graph = os.environ.get('MRGP_SHARDED_GRAPH', '1') != '0'
-        if not use_graph:
-            with torch.cuda.stream(self.stream):
-                for _ in range(n_iter):
-                    self._sweep_body()
-            return
-        if self._graph is None:
-            with torch.cuda.stream(self.stream):
-                self._sweep_body()                       # warm-up outside capture (NCCL lazy init)
-            self.stream.synchronize()
-            n_iter -= 1
-            self._graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(self._graph, stream=self.stream):
-                self._sweep_body()
-            # capture records, it does not execute
-        for _ in range(n_iter):
-            with torch.cuda.stream(self.stream):
-                self._graph.replay()
+        if use_graph:
+            self._ck(self.lib.mrgp_sweep(self.handle, int(n_iter)))
+        else:
+            for _ in range(n_iter):
+                self.sweep_stepwise()
 
     def latent(self, j):
         raise NotImplementedError('latent export is not available on a sharded engine')

@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define MRGP_ABI_VERSION 4
+#define MRGP_ABI_VERSION 5
 
 enum {
     MRGP_OK = 0,
@@ -259,24 +259,18 @@ int mrgp_predict_var_indexed(mrgp_handle *h, const double *x_test_dev, int64_t n
  * LOCAL rows) but knows every region.  The per-region sufficient statistics of a phase (<= R x 60 doubles) are
  * summed over the ranks and consumed by the replicated small-matrix step; no per-sample data ever leaves a GPU.
  *
- * (1) Peer-memory exchange (the product path): every rank keeps a small arena that the peers map over
- *     NVLink / NVSwitch (CUDA IPC between processes, plain pointers inside one process).
- *         mrgp_comm_export(h, blob)                     -> 128-byte description of this rank's arena
- *         (all-gather the blobs of all ranks with any transport: torch.distributed, MPI, a file)
- *         mrgp_comm_bind(h, rank, world, blobs, bounds) -> maps the peers; bounds[q], bounds[q+1] = samples of rank q
- *     Afterwards mrgp_build_basis, mrgp_sweep (one CUDA graph, exchanges included) and mrgp_exchange work on the
- *     sharded handle.  One exchange = dense local sums -> arena, a release-store of the next sequence number into
- *     every peer's flag array, and a reduce kernel that waits for all peers and sums, per region, the arenas of
- *     exactly the ranks that own samples of the region, in rank order: every rank computes bit-identical sums.
- *     A peer that never publishes makes the wait time out (15 s) and mrgp_synchronize return MRGP_ECUDA.
- *         mrgp_phase_a -> mrgp_exchange(layer, MRGP_X_PHASE_A) -> mrgp_axis_update
- *         mrgp_phase_b -> mrgp_exchange(layer, MRGP_X_PHASE_B) -> mrgp_bias_noise
- * (2) Caller-side collective (NCCL all-reduce on the handle's stream; kept as the comparison arm):
- *         mrgp_phase_a -> mrgp_region_sums(layer, MRGP_X_PHASE_A) -> all-reduce SUM -> mrgp_axis_update
- *         mrgp_phase_b -> mrgp_region_sums(layer, MRGP_X_PHASE_B) -> all-reduce SUM -> mrgp_bias_noise
- *     and at construction
- *         mrgp_build_basis_stage(layer, 0) -> all-reduce MAX -> stage 1 -> all-reduce SUM -> stage 2.
- *     mrgp_sweep() is refused on a sharded handle without (1).                                            */
+ * The sums go through a peer-memory exchange: every rank keeps a small arena that the peers map over
+ * NVLink / NVSwitch (CUDA IPC between processes, plain pointers inside one process).
+ *     mrgp_comm_export(h, blob)                     -> 128-byte description of this rank's arena
+ *     (all-gather the blobs of all ranks with any transport: torch.distributed, MPI, a file)
+ *     mrgp_comm_bind(h, rank, world, blobs, bounds) -> maps the peers; bounds[q], bounds[q+1] = samples of rank q
+ * Afterwards mrgp_build_basis, mrgp_sweep (one CUDA graph, exchanges included) and mrgp_exchange work on the
+ * sharded handle; before it they are refused.  One exchange = dense local sums -> arena, a release-store of the next
+ * sequence number into every peer's flag array, and a reduce kernel that waits for all peers and sums, per region,
+ * the arenas of exactly the ranks that own samples of the region, in rank order: every rank computes bit-identical
+ * sums.  A peer that never publishes makes the wait time out (15 s) and mrgp_synchronize return MRGP_ECUDA.
+ *     mrgp_phase_a -> mrgp_exchange(layer, MRGP_X_PHASE_A) -> mrgp_axis_update
+ *     mrgp_phase_b -> mrgp_exchange(layer, MRGP_X_PHASE_B) -> mrgp_bias_noise                                */
 enum { MRGP_X_PHASE_A = 0, MRGP_X_PHASE_B = 1 };
 #define MRGP_COMM_BLOB_BYTES 128
 #define MRGP_COMM_MAX_RANKS 16
@@ -287,9 +281,6 @@ int mrgp_exchange(mrgp_handle *h, int32_t layer, int32_t which);
  * N = 1e6).  With them every rank builds the basis invariants of the closed-form statistics (DESIGN.md §4) and
  * the layers above the first need neither their samples nor an exchange in mrgp_sweep.  y never leaves its rank. */
 int mrgp_set_all_inputs_host(mrgp_handle *h, const double *x_all_host);
-int mrgp_region_sums(mrgp_handle *h, int32_t layer, int32_t which);
-int mrgp_exchange_buffer(mrgp_handle *h, int32_t layer, int32_t which, void **dev_ptr, size_t *n_doubles);
-int mrgp_build_basis_stage(mrgp_handle *h, int32_t layer, int32_t stage, double interval_factor);
 
 /* ---- groups of independent models (BASELINE config 5: a batch of series) --------------------------------- */
 

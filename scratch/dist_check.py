@@ -17,14 +17,14 @@ n,res,M=int(os.environ.get('MRGP_N','200000')),7,30
 x,y=workloads.workload1(n); xs=(x-x.mean(0))/x.std(0); offs=O.uniform_offsets(n,res,2)
 t=time.time()
 e=ShardedEngine(xs,y,offs,M,rank,world,device=lr)
-print('rank',rank,e.exchange,'built %.2fs'%(time.time()-t),flush=True)
+print('rank',rank,'built %.2fs'%(time.time()-t),flush=True)
 t=time.time(); e.sweep(2,use_graph=False); e.synchronize(); print('rank',rank,'2 stepwise sweeps ok %.2fs'%(time.time()-t),flush=True)
 t=time.time(); e.sweep(3); e.synchronize(); print('rank',rank,'3 graph sweeps ok %.2fs'%(time.time()-t),flush=True)
 ref=Engine(xs,y,offs,M,device=lr); ref.sweep(5); ref.synchronize()
 a,b=e.state(),ref.state(latent=False)
 worst=max(float(np.max(np.abs(a[k]-b[k])/(np.abs(b[k])+1e-12*np.abs(b[k]).max()+1e-300))) for k in b)
 print('rank',rank,'max rel diff vs unsharded %.2e'%worst,flush=True)
-if e.exchange=='peer' and not one:
+if not one:
     ev0,ev1=torch.cuda.Event(enable_timing=True),torch.cuda.Event(enable_timing=True)
     e.sweep(5); e.synchronize(); dist.barrier()
     ev0.record(e.stream); e.sweep(20); ev1.record(e.stream); e.synchronize()

@@ -22,7 +22,7 @@ class TC(object):
 
 if warm1:
     c1 = TC(1); c1.local.rank = 0
-    e1 = ShardedEngine(xs, y, offs, M, 0, 1, comm=c1, exchange='peer'); e1.sweep(2); e1.sweep(1, use_graph=False); e1.synchronize()
+    e1 = ShardedEngine(xs, y, offs, M, 0, 1, comm=c1); e1.sweep(2); e1.sweep(1, use_graph=False); e1.synchronize()
     a, b = e1.state(), ref.state(latent=False)
     print('world-1 sharded max rel diff %.2e' % max(float(np.max(np.abs(a[k]-b[k])/(np.abs(b[k])+1e-12*np.abs(b[k]).max()+1e-300))) for k in b), flush=True)
 comm = TC(world); engines = [None] * world
@@ -30,7 +30,7 @@ def work(rank):
     comm.local.rank = rank
     t0 = time.time()
     try:
-        e = ShardedEngine(xs, y, offs, M, rank, world, comm=comm, exchange='peer')
+        e = ShardedEngine(xs, y, offs, M, rank, world, comm=comm)
         print(rank, 'built %.2fs' % (time.time() - t0), flush=True)
         if os.environ.get('GRAPH','1')=='1':
             e.sweep(2); e.synchronize(); print(rank, 'graph sweeps ok %.2fs' % (time.time() - t0), flush=True)

@@ -52,7 +52,7 @@ def run(root, out):
         e.synchronize()
         for k, v in e.state(latent=False).items():
             res['%s/%s' % (name, k)] = v
-        if elbo:
+        if elbo and e.mode == 'ci':   # the library defines the bound in ci mode only
             res[name + '/elbo'] = e.elbo()
         res[name + '/launches'] = np.array([e.launch_count()])
         print(name, 'launches', e.launch_count(), flush=True)
@@ -148,10 +148,10 @@ def run(root, out):
         def work(rank):
             comm.local.rank = rank
             try:
-                e = ShardedEngine(normed(x), y, offs, 30, rank, 2, comm=comm, exchange='peer', mode=mode)
-                e.sweep(2)
-                e.synchronize()
-                e.sweep(1, use_graph=False)
+                e = ShardedEngine(normed(x), y, offs, 30, rank, 2, comm=comm, mode=mode)
+                # phase by phase, as in test_sample_sharding_matches_single_handle: with both ranks in one process on
+                # one device the captured sweep's exchanges time out; the captured form is checked between processes
+                e.sweep(3, use_graph=False)
                 e.synchronize()
                 engines[rank] = e
             except Exception as ex:

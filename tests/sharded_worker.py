@@ -27,7 +27,7 @@ n, res, M = 30000, 6, 30
 x, y = workloads.workload1(n)
 xs = (x - x.mean(0)) / x.std(0)
 offsets = O.uniform_offsets(n, res, 2)
-e = ShardedEngine(xs, y, offsets, M, rank, world, exchange='peer', mode=mode, device=0)
+e = ShardedEngine(xs, y, offsets, M, rank, world, mode=mode, device=0)
 e.sweep(1, use_graph=False)          # phase by phase through mrgp_exchange
 e.sweep(2)                           # one captured CUDA graph per sweep, exchanges inside
 e.synchronize()

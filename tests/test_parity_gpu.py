@@ -301,26 +301,13 @@ def test_constructor_errors_match_reference():
 
 
 class _ThreadComm(object):
-    """In-process stand-in for the NCCL all-reduce: the ranks are Python threads driving their own handle (all on
-    cuda:0); tensors are summed through host-synchronised device ops."""
+    """In-process stand-in for torch.distributed: the ranks are Python threads driving their own handle (all on
+    cuda:0); the arena descriptions are gathered through a shared list."""
 
     def __init__(self, world):
         import threading
         self.world, self.slots, self.barrier = world, [None] * world, threading.Barrier(world)
         self.local = threading.local()
-
-    def all_reduce(self, tensor, op):
-        import torch
-        torch.cuda.synchronize()
-        self.slots[self.local.rank] = tensor
-        self.barrier.wait()
-        stack = torch.stack([t for t in self.slots])
-        res = stack.max(0).values if op == 'max' else stack.sum(0)
-        torch.cuda.synchronize()
-        self.barrier.wait()
-        tensor.copy_(res)
-        torch.cuda.synchronize()
-        self.barrier.wait()
 
     def all_gather_bytes(self, payload):
         self.slots[self.local.rank] = bytes(payload)
@@ -333,12 +320,12 @@ class _ThreadComm(object):
         self.barrier.wait()
 
 
-@pytest.mark.parametrize('fi,world,exchange', [(False, 2, 'nccl'), (True, 3, 'nccl'), (False, 3, 'peer'), (True, 2, 'peer')])
-def test_sample_sharding_matches_single_handle(fi, world, exchange):
+@pytest.mark.parametrize('fi,world', [(False, 2), (True, 3), (False, 3), (True, 2)])
+def test_sample_sharding_matches_single_handle(fi, world):
     """The multi-GPU decomposition (sample chunks + summed region statistics) on one device: every rank must
-    end with the state of the unsharded run (up to the summation order of the exchanged statistics).  'peer':
-    the library's own exchange through mapped arenas (here: handles of one process, plain pointers), driven phase
-    by phase (the captured-graph form runs between processes, next test); 'nccl': the caller-side all-reduce arm."""
+    end with the state of the unsharded run (up to the summation order of the exchanged statistics).  The
+    statistics go through the library's own exchange over mapped arenas (here: handles of one process, plain
+    pointers), driven phase by phase (the captured-graph form runs between processes, next test)."""
     import threading
     from cimrgp_b200.distributed import ShardedEngine, chunk_bounds
     from cimrgp_b200.engine import Engine
@@ -356,7 +343,7 @@ def test_sample_sharding_matches_single_handle(fi, world, exchange):
     def work(rank):
         try:
             comm.local.rank = rank
-            e = ShardedEngine(xs, y, offsets, M, rank, world, comm=comm, exchange=exchange, mode=mode)
+            e = ShardedEngine(xs, y, offsets, M, rank, world, comm=comm, mode=mode)
             for _ in range(3):
                 e.sweep(1, use_graph=False)
             e.synchronize()
@@ -378,7 +365,7 @@ def test_sample_sharding_matches_single_handle(fi, world, exchange):
         assert np.array_equal(a[k], b[k]), k     # replicated small-matrix steps: identical on every rank
 
 
-@pytest.mark.parametrize('mode,world', [('ci', 2), ('fi', 3)])
+@pytest.mark.parametrize('mode,world', [('ci', 2), ('fi', 3), ('ci', 3), ('fi', 2)])
 def test_peer_exchange_between_processes(mode, world):
     """The product form of the multi-GPU path: one process per rank, arenas mapped through CUDA IPC, the sweep one
     CUDA graph with the exchanges inside.  The ranks share cuda:0 here (the parity box has one GPU)."""
